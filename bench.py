@@ -343,6 +343,41 @@ def fp64_gemm_peak():
     return best
 
 
+P_SAMPLE, DUMP_SEED = 1 << 20, 2024
+
+
+def filter_outputs(g, b=0, prefix=""):
+    """what a caller of rslam_frame receives for filter b after a frame: the state x, the covariance P, the per-feature predictions,
+    matches and inlier flags, and the RANSAC result.  A P of more than 2^20 entries (1.15 GB at C3) is given by its diagonal, its 13
+    camera rows and a fixed sample of 2^20 entries drawn with DUMP_SEED (flat column-major indices in P_sample_index)."""
+    x, P = g.download_state(b=b)
+    n = x.size
+    out = dict(x=x)
+    if n * n <= P_SAMPLE:
+        out["P"] = P
+    else:
+        flat = np.random.default_rng(DUMP_SEED).integers(0, n * n, P_SAMPLE)
+        out.update(P_diag=np.diag(P).copy(), P_camera_rows=np.ascontiguousarray(P[:13]), P_sample=P.reshape(-1, order="F")[flat],
+                   P_sample_index=flat.astype(np.float64))
+    ft = g.features(b)
+    out.update(h=ft["h"], S=ft["S"], z=ft["z"])
+    for k in ("has_h", "ic", "li", "hi", "times_predicted", "times_measured"):
+        out[k] = ft[k].astype(np.float32)
+    r = g.ransac_result(b)
+    out["ransac"] = np.array([r[k] for k in ("status", "hyp_run", "best_support", "n_hyp", "num_ic", "winner")], dtype=np.float64)
+    return {prefix + k: v for k, v in out.items()}
+
+
+def dump_outputs(directory, arrays):
+    """arrays: name -> float32 / float64 array, written as directory/<name>.npy"""
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"{total} bytes of outputs, more than 64 MB"
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def frame_stats(g, b=0):
     ft = g.features(b)
     r = g.ransac_result(b)
@@ -590,6 +625,8 @@ def bench_c3(args, world, rank, local):
     value = K / (ms * 1e-3)
     pose_resident = g.download_pose()
     st_last = frame_stats(g)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, filter_outputs(g))
     # ---- per-kernel breakdown: instrumented pass (CUDA events around every launch on the launching stream, no graph) on the next frames
     g.profile(True)
     stats = []
@@ -667,8 +704,9 @@ def bench_c3(args, world, rank, local):
 # ---------------------------------------------------------------------------------------------------------------------
 # --gpus N > 1 (and a "workloads" entry at N = 1): C5, independent 100-feature filters split over the ranks, no collective
 # ---------------------------------------------------------------------------------------------------------------------
-def bench_c5(args, world, rank, local, filters_total=None, steps=None, warmup=None, with_e2e=True, ranks_active=None):
-    """ranks_active: run on the first `ranks_active` ranks only (the others idle): the same-run single-GPU figure of the scaling line"""
+def bench_c5(args, world, rank, local, filters_total=None, steps=None, warmup=None, with_e2e=True, ranks_active=None, dump_dir=None):
+    """ranks_active: run on the first `ranks_active` ranks only (the others idle): the same-run single-GPU figure of the scaling line.
+    dump_dir: rank 0 writes the outputs of 8 of its filters, evenly spaced over its batch, after the last timed step"""
     import torch
 
     from ransac_slam_b200 import capi
@@ -719,6 +757,11 @@ def bench_c5(args, world, rank, local, filters_total=None, steps=None, warmup=No
     launches = g.launches - l0
     clocks = sampler.stop() if rank == 0 else None
     pose_resident = g.download_pose(b=Bl - 1)
+    if dump_dir and rank == 0:
+        arrays = {}
+        for b in np.unique(np.linspace(0, Bl - 1, 8).astype(int)):
+            arrays.update(filter_outputs(g, b=int(b), prefix=f"filter{b}_"))
+        dump_outputs(dump_dir, arrays)
     # instrumented pass (events around every launch, no graph): where the batch frame goes
     g.profile(True)
     run_frames_resident(g, d_images, d_u01, [W + K], False, None, stream)
@@ -795,7 +838,7 @@ def c5_line(args, world, rank, local):
     single = bench_c5(args, world, rank, local, steps=min(args.steps, 6), warmup=3, with_e2e=False, ranks_active=1)
     barrier(world)
     torch.cuda.empty_cache()
-    r = bench_c5(args, world, rank, local)
+    r = bench_c5(args, world, rank, local, dump_dir=args.dump_outputs)
     barrier(world)
     ms = max_over_ranks(r["ms"], world)
     K, W = r["steps"], r["warmup"]
@@ -880,7 +923,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--extras", default="c2,c4,c5")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, at most 64 MB), "
+                                                         "to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     # stdout carries exactly ONE line, the JSON: everything libraries print while we run (NCCL's version banner ...) goes to stderr

@@ -11,6 +11,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_PATH = os.path.join(_HERE, "_build", "liborc.so")
+_SHIM_PATH = os.path.join(_HERE, "_build", "libshim.so")
 
 Q1 = 1 << 0  # angles taken from the position vector (src/Tracking.cpp:448)
 Q4 = 1 << 1  # pow(s, -3/2) -> s^-1 (src/ExtendKF.cpp:627)
@@ -20,8 +21,9 @@ Q_ALL = 0xF
 
 
 def build(force=False):
-    srcs = [os.path.join(_HERE, f) for f in ("rslam_oracle.cpp", "gemm.cpp", "omat.h", "Makefile")]
-    if (not force) and os.path.exists(_LIB_PATH) and all(os.path.getmtime(_LIB_PATH) >= os.path.getmtime(s) for s in srcs):
+    srcs = [os.path.join(_HERE, f) for f in ("rslam_oracle.cpp", "gemm.cpp", "omat.h", "shim_probe.cpp", "ref_shim/mini_eigen.h", "ref_shim/mini_cv.h",
+                                             "Makefile")]
+    if (not force) and all(os.path.exists(out) and all(os.path.getmtime(out) >= os.path.getmtime(s) for s in srcs) for out in (_LIB_PATH, _SHIM_PATH)):
         return _LIB_PATH
     subprocess.check_call(["make", "-C", _HERE, "all"], stdout=subprocess.DEVNULL)
     return _LIB_PATH
@@ -73,6 +75,12 @@ def lib():
         _lib.orc_get_types.argtypes = [C.c_void_p, C.c_void_p]
         _lib.orc_get_feature_init.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     return _lib
+
+
+def shim_lib():
+    """oracle/_build/libshim.so: the stand-in Eigen / OpenCV headers of ref_shim/ behind C entry points (shim_probe.cpp)"""
+    build()
+    return C.CDLL(_SHIM_PATH)
 
 
 def _p(a):

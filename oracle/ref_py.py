@@ -3,7 +3,7 @@ the stand-in Eigen / OpenCV / ROS headers of oracle/ref_shim/) behind oracle/ref
 
 It can be BUILT only where /root/reference exists (the build container: `make -C oracle ref`, done by __graft_entry__.build()); the
 GPU box gets the prebuilt, git-ignored .so with the snapshot.  `available()` says whether the library is there; the committed golden
-vectors it produced (tests/golden/ref_vectors.npz, tests/golden/make_ref_vectors.py) cover the case where it is not.
+vectors it produced (tests/golden/ref_vectors.*.npz, tests/golden/make_ref_vectors.py) cover the case where it is not.
 """
 import ctypes as C
 import os

@@ -1,5 +1,5 @@
 """The full-size configuration C3 (N = 2000 features, state dimension 12013, P = 1.15 GB) as a deterministic test case: inputs built
-with element-wise numpy only, so that the committed outputs of the CPU oracle (tests/golden/c3_vectors.npz, written by
+with element-wise numpy only, so that the committed outputs of the CPU oracle (tests/golden/c3_vectors.*.npz, written by
 tests/golden/make_c3_vectors.py) belong to exactly the inputs the GPU test rebuilds on the box."""
 import hashlib
 

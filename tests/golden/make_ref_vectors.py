@@ -1,4 +1,4 @@
-"""Generates tests/golden/ref_vectors.npz from the REFERENCE'S OWN SOURCES (oracle/_ref/libref.so = /root/reference/src/{ExtendKF,
+"""Generates tests/golden/ref_vectors.*.npz from the REFERENCE'S OWN SOURCES (oracle/_ref/libref.so = /root/reference/src/{ExtendKF,
 Tracking,Converter,Map}.cpp compiled unmodified against the stand-in third-party headers of oracle/ref_shim/, see
 oracle/ref_driver.cpp).  Run in the build container, where /root/reference exists:
 
@@ -20,6 +20,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import ref_py as R  # noqa: E402
+from tests import golden_npz  # noqa: E402
 from tests import helpers as H  # noqa: E402
 
 BUNDLED_FRAMES = 9          # frames 7 and 8 run Map::map_management's delete pass (12 and 8 deletions, run-ahead index, src/Map.cpp:19-32)
@@ -193,6 +194,5 @@ if __name__ == "__main__":
     bundled(out)
     q1(out)
     convert(out)
-    path = os.path.join(ROOT, "tests", "golden", "ref_vectors.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+    for path in golden_npz.save("ref_vectors", out):
+        print("wrote", path, os.path.getsize(path) // 1024, "KiB")

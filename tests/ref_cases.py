@@ -1,10 +1,11 @@
-"""The three cases of tests/golden/ref_vectors.npz (produced by the REFERENCE'S OWN SOURCES, see tests/golden/make_ref_vectors.py),
+"""The three cases of tests/golden/ref_vectors.*.npz (produced by the REFERENCE'S OWN SOURCES, see tests/golden/make_ref_vectors.py),
 written once against a tiny engine interface so that the CPU oracle and the CUDA path (through the C ABI) are both checked against
 the same reference outputs.  Bars (north_star): flags / match indices / hypothesis counts bit-exact, x and P within 1e-9 relative."""
 import os
 
 import numpy as np
 
+from tests import golden_npz
 from tests import helpers as H
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -12,7 +13,7 @@ RAND_MAX = 2147483647
 
 
 def load():
-    return np.load(os.path.join(GOLD, "ref_vectors.npz"))
+    return golden_npz.load("ref_vectors")
 
 
 def u01_of(draws):
@@ -194,7 +195,7 @@ def run_bundled(make_engine, frames=None):
         e.update_hi()
         x, P = e.state()
         H.assert_x_close(x, g[pre + "x"], what=f"{e.name}: x after frame {k}")
-        if pre + "P" in g.files:
+        if pre + "P" in g:
             H.assert_P_close(P, g[pre + "P"], what=f"{e.name}: P after frame {k}")
         else:  # later frames store diag(P) and four fixed projections P v instead of the whole matrix
             V = np.random.default_rng(1000 + k).standard_normal((P.shape[0], 4))

@@ -3,7 +3,7 @@
   C3  one whole frame of the 2000-feature filter (state dimension 12013, P 1.15 GB) against the CPU oracle in sparse mode -- match
       lists, RANSAC replay (hyp_run, n_hyp, support), li / hi sets bit for bit; x and P to 1e-9 -- with the reference's quirks on (one
       low-innovation inlier, ~1990 rescued ones: the joint update at k ~ 3980 through k_chol_panel / k_trsm_ll / k_gemm_dmma) and
-      with Q1 off (a real low-innovation set).  The oracle's outputs are the committed fixture tests/golden/c3_vectors.npz
+      with Q1 off (a real low-innovation set).  The oracle's outputs are the committed fixture tests/golden/c3_vectors.*.npz
       (tests/golden/make_c3_vectors.py; the inputs are rebuilt here bit for bit, checked by a digest); RSLAM_LIVE_ORACLE=1 re-runs
       the oracle on the box instead (~3 minutes per case on 8 cores).
   C4  the support sweep over 5000 matches (state dimension 30013, P 7.2 GB): 200 hypotheses against a numpy restatement of
@@ -19,11 +19,11 @@ import pytest
 from oracle import np_oracle as NP
 from ransac_slam_b200 import synth, sweep
 from tests import c3_case as C3
+from tests import golden_npz
 from oracle import oracle_py as O
 from tests import helpers as H
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 _c3_cache = {}
 
@@ -43,9 +43,9 @@ def test_c3_whole_frame_vs_oracle(tag, quirks):
     live = os.environ.get("RSLAM_LIVE_ORACLE", "0") == "1"
     exp = None
     if not live:
-        g = np.load(os.path.join(GOLD, "c3_vectors.npz"))
+        g = golden_npz.load("c3_vectors")
         if str(g["digest"]) == C3.input_digest(scene, seq, P0):
-            exp = {k[len(tag) + 1:]: g[k] for k in g.files if k.startswith(tag + "_")}
+            exp = {k[len(tag) + 1:]: g[k] for k in g if k.startswith(tag + "_")}
     if exp is None:  # inputs differ on this machine (libm / numpy build): run the oracle here
         exp = C3.run_oracle(quirks, cam, scene, seq, P0)
     f = capi.Filter(cam.as9(), C3.N, quirks=quirks, std_a=0.007 * C3.STD_SCALE, std_alpha=0.007 * C3.STD_SCALE)

@@ -1,4 +1,4 @@
-"""Configuration C1 on the device: all 100 frames of the reference's bundled sequence (tests/golden/pgm_frames_all.npz) through the C++ host
+"""Configuration C1 on the device: all 100 frames of the reference's bundled sequence (tests/golden/pgm_frames_all.*.npz) through the C++ host
 classes in System::TrackRunning's order (rslam_replay_pgm), with the libc draws of tests/golden/c1_ref_outputs.npz, against
   * the outputs of the reference's OWN sources on the same frames and draws (tools/c1_replay.py ref) for as long as the reference is
     defined: 37 frames.  At frame 37 the warped window of one feature is 13 x 12 (cv::Range truncates toward zero, quirk Q13) and

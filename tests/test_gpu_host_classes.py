@@ -51,7 +51,7 @@ def test_host_classes_replay(tmp_path):
 def test_pgm_replay_through_host_classes_matches_the_reference(tmp_path):
     """configuration C1 end to end: frames of the reference's bundled sequence written as P5 files, replayed by the C++ drop-in
     classes in System::System / System::TrackRunning order (rslam_replay_pgm), against the outputs of the reference's own sources
-    (tests/golden/ref_vectors.npz) fed the same libc draws."""
+    (tests/golden/ref_vectors.*.npz) fed the same libc draws."""
     from oracle import ref_py as R  # only for the settings template (numbers of examples/Monocular/initialize_param.yaml)
     from tests import ref_cases as RC
 

@@ -335,8 +335,6 @@ def test_patch_warp_matches_oracle_remap():
         worst = max(worst, float(d.max()))
     stats = f"patch warp vs oracle: {same}/{int(fo['has_h'].sum())} patches identical, {neq}/{npix} pixels identical, max |d| = {worst}"
     print(stats)
-    if os.path.isdir("gpurun_out"):
-        open("gpurun_out/r02_patch_stats.txt", "a").write(stats + "\n")
     assert neq >= npix - 2, stats  # bit-identical pixels (a flip needs a coordinate within ~1e-13 px of a quantisation boundary)
     # build an image that contains the oracle-predicted appearance at a pasted location and search on both sides
     img = synth.background(scene.cam).copy()

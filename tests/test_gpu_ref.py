@@ -1,4 +1,4 @@
-"""CUDA path (through the C ABI) against outputs of the REFERENCE'S OWN SOURCES (tests/golden/ref_vectors.npz, produced by
+"""CUDA path (through the C ABI) against outputs of the REFERENCE'S OWN SOURCES (tests/golden/ref_vectors.*.npz, produced by
 oracle/_ref/libref.so: /root/reference/src/*.cpp compiled unmodified, see tests/golden/make_ref_vectors.py and tests/test_ref_pin.py).
 Bars: flags, match pixels, FAST corners and hypothesis counts bit-exact; x and P within 1e-9 relative."""
 import numpy as np

@@ -1,6 +1,6 @@
 """Pins the CPU oracle to the REFERENCE'S OWN SOURCES.
 
-tests/golden/ref_vectors.npz holds outputs of /root/reference/src/{ExtendKF,Tracking,Converter,Map}.cpp, compiled unmodified
+tests/golden/ref_vectors.*.npz holds outputs of /root/reference/src/{ExtendKF,Tracking,Converter,Map}.cpp, compiled unmodified
 (oracle/Makefile `ref`, stand-in Eigen / OpenCV / ROS headers in oracle/ref_shim/) and driven through the reference's own
 TrackRunning call sequence.  The oracle must reproduce them: flags, match pixels and hypothesis counts exactly, x and P to 1e-9.
 Where oracle/_ref/libref.so is present (the build container; the GPU box when the prebuilt library travelled) the live library is
@@ -116,13 +116,12 @@ def test_distortion_model_matches_live_reference():
     assert np.array_equal(o.undistort(uv), r.undistort(uv))
 
 
-# ---- the stand-in third-party headers themselves (oracle/ref_shim/) ---------------------------------------------------------------
-@needs_ref
+# ---- the stand-in third-party headers themselves (oracle/ref_shim/, through oracle/shim_probe.cpp) --------------------------------------
 def test_shim_opencv_primitives_match_cv2_fixtures():
-    """mini_cv.h's remap / calcCovarMatrix (through the reference's own Converter::corrcoef_opencv) / FAST against cv2 4.13 outputs"""
+    """mini_cv.h's remap / calcCovarMatrix / FAST against cv2 4.13 outputs"""
     import ctypes as C
 
-    L = R.lib()
+    L = O.shim_lib()
     fx = np.load(os.path.join(RC.GOLD, "cv_fixtures.npz"))
     for k in range(6):
         src = np.ascontiguousarray(fx[f"remap_src_{k}"], np.float32)
@@ -133,12 +132,12 @@ def test_shim_opencv_primitives_match_cv2_fixtures():
                        C.c_int(mx.shape[0]), C.c_int(mx.shape[1]), out.ctypes.data_as(C.c_void_p))
         assert np.array_equal(out, fx[f"remap_dst_{k}"]), k
     for k in range(3):
-        M = np.ascontiguousarray(fx[f"covar_M_{k}"], np.float64)
+        M = np.ascontiguousarray(fx[f"covar_M_{k}"], np.float32)
         cov = fx[f"covar_cov_{k}"]
-        want = cov / np.sqrt(np.outer(np.diag(cov), np.diag(cov)))
         got = np.zeros((M.shape[1], M.shape[1]))
-        L.ref_corrcoef_opencv(M.ctypes.data_as(C.c_void_p), C.c_int(M.shape[0]), C.c_int(M.shape[1]), got.ctypes.data_as(C.c_void_p))
-        np.testing.assert_allclose(got, want, rtol=0, atol=5e-15)
+        L.ref_cv_calc_covar(M.ctypes.data_as(C.c_void_p), C.c_int(M.shape[0]), C.c_int(M.shape[1]), got.ctypes.data_as(C.c_void_p))
+        scale = np.sqrt(np.outer(np.diag(cov), np.diag(cov)))  # the correlation matrix Converter::corrcoef_opencv makes of it
+        np.testing.assert_allclose(got / scale, cov / scale, rtol=0, atol=5e-15)
     ff = np.load(os.path.join(RC.GOLD, "fast_fixtures.npz"))
     total = 0
     for name in ff["names"]:
@@ -153,13 +152,12 @@ def test_shim_opencv_primitives_match_cv2_fixtures():
     assert total > 300
 
 
-@needs_ref
 def test_shim_eigen_semantics_match_numpy():
-    """the Eigen behaviours the reference's sources rely on, as mini_eigen.h implements them, against numpy (oracle/ref_driver.cpp:
+    """the Eigen behaviours the reference's sources rely on, as mini_eigen.h implements them, against numpy (oracle/shim_probe.cpp:
     ref_eigen_probe lists them; the first is the row-by-row comma initialiser behind quirk Q16)"""
     import ctypes as C
 
-    L = R.lib()
+    L = O.shim_lib()
     n = 6
     rng = np.random.default_rng(12)
     A = np.asfortranarray(rng.uniform(0.1, 1.0, (n, n)) + 2.0 * np.eye(n))

@@ -5,7 +5,7 @@ replayed in sorted order through System::TrackRunning's call sequence with the l
   python tools/c1_replay.py ref   [--out tests/golden/c1_ref_outputs.npz]   reference's own sources (oracle/_ref/libref.so), CPU, here
   python tools/c1_replay.py gpu                                              rslam_replay_pgm (C++ host classes over the C ABI), GPU box
 Both print one JSON line with frames/s and the per-frame feature / match / inlier counts; `gpu` also compares with the committed reference
-outputs frame by frame.  Frames come from /root/reference when it exists, else from tests/golden/pgm_frames_all.npz."""
+outputs frame by frame.  Frames come from /root/reference when it exists, else from tests/golden/pgm_frames_all.*.npz."""
 import json
 import os
 import subprocess
@@ -44,7 +44,9 @@ def load_frames():
     if os.path.isdir(SEQ):
         names = sorted(f for f in os.listdir(SEQ) if f.endswith(".pgm"))
         return np.stack([read_pgm(os.path.join(SEQ, f)) for f in names]), names
-    g = np.load(os.path.join(GOLD, "pgm_frames_all.npz"))
+    from tests import golden_npz
+
+    g = golden_npz.load("pgm_frames_all")
     return g["frames"], [str(s) for s in g["names"]]
 
 
