@@ -118,6 +118,13 @@ def ekf_update(x, P, H, z, h, q4_int_exponent=True):
     xkk = x + K @ (z - h)
     Pt = P - K @ S @ K.T
     Pk = 0.5 * Pt + 0.5 * Pt.T
+    return normalise_quaternion(xkk, Pk, q4_int_exponent)
+
+
+def normalise_quaternion(xkk, Pk, q4_int_exponent=True):
+    """The quaternion normalisation that closes ExtendKF::update (src/ExtendKF.cpp:611-634): x_k_k[3:7] / |q| and
+    P <- Tm P Tm^T with Tm the identity except for Jn in rows / columns 3..6.  Tm is applied to those four rows and columns only
+    (O(n) instead of two dense n^3 products)."""
     r, qx, qy, qz = xkk[3:7]
     s = r * r + qx * qx + qy * qy + qz * qz
     T = np.array([[qx * qx + qy * qy + qz * qz, -r * qx, -r * qy, -r * qz], [-qx * r, r * r + qy * qy + qz * qz, -qx * qy, -qx * qz],
@@ -125,10 +132,10 @@ def ekf_update(x, P, H, z, h, q4_int_exponent=True):
     Jn = (s ** -1.0 if q4_int_exponent else s ** -1.5) * T
     xkk = xkk.copy()
     xkk[3:7] = xkk[3:7] / np.sqrt(s)
-    n = x.size
-    Tm = np.eye(n)
-    Tm[3:7, 3:7] = Jn
-    return xkk, Tm @ Pk @ Tm.T
+    Pn = np.array(Pk, copy=True)
+    Pn[3:7, :] = Jn @ Pn[3:7, :]
+    Pn[:, 3:7] = Pn[:, 3:7] @ Jn.T
+    return xkk, Pn
 
 
 def hypothesis_support(cam, x, P, types, H_p, h_p, z_p, z_all, has_z, std_z=1.0, q1=True):

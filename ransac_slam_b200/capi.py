@@ -234,6 +234,13 @@ class Filter:
         self._ck(self.L.rslam_download_H(self.h, b, _p(Hc), _p(Hf)))
         return Hc, Hf
 
+    def upload_linearisation(self, h, Hc, Hf, z, flags, b=0):
+        """Caller-built linearisation of filter b (ExtendKF::update with its own H, z, h): h, z (N, 2); Hc (N, 2, 7); Hf (N, 2, 6), of which
+        a cartesian feature uses columns 0..2; flags (N, 4) = has_h, ic, li, hi.  The next update_li / update_hi runs on it."""
+        arrs = [np.ascontiguousarray(v, dtype=np.float64) for v in (h, Hc, Hf, z)]
+        fl = np.ascontiguousarray(flags, dtype=np.uint8)
+        self._ck(self.L.rslam_upload_linearisation(self.h, b, *[_p(v) for v in arrs], _p(fl)))
+
     def set_matches(self, z, ic, b=0):
         z = np.ascontiguousarray(z, dtype=np.float64)
         ic = np.ascontiguousarray(ic, dtype=np.uint8)

@@ -353,8 +353,6 @@ def test_patch_warp_matches_oracle_remap():
 def test_upload_linearisation_reproduces_the_update_and_stage_entry_points():
     """rslam_upload_linearisation (what the host ExtendKF::update uses when it is handed caller-built H, z, h) and the two halves of
     search_IC_matches as separate entry points (Tracking::calculate_derivatives / matching)."""
-    import ctypes as C
-
     scene, x, P = synth.random_spd_state(40, seed=131)
     seq = synth.make_sequence(scene, T=1, seed=136, t0=3)
     a = H.gpu_from(scene, x, P, quirks=0x6)
@@ -374,9 +372,7 @@ def test_upload_linearisation_reproduces_the_update_and_stage_entry_points():
     fb = b.features()
     assert (fb["ic"] == fa["ic"]).all() and np.array_equal(fb["z"][fb["ic"]], fa["z"][fa["ic"]]) and np.array_equal(fb["h"], fa["h"])
     flags = np.stack([fa["has_h"], fa["ic"], fa["li"], np.zeros_like(fa["li"])], axis=1).astype(np.uint8)
-    arrs = [np.ascontiguousarray(v, dtype=np.float64) for v in (fa["h"], Hc, Hf, fa["z"])]
-    rc = L.rslam_upload_linearisation(b.h, 0, *[v.ctypes.data_as(C.c_void_p) for v in arrs], np.ascontiguousarray(flags).ctypes.data_as(C.c_void_p))
-    assert rc == 0
+    b.upload_linearisation(fa["h"], Hc, Hf, fa["z"], flags)
     b.update_li()
     xb, Pb = b.download_state()
     assert np.array_equal(xa, xb) and np.array_equal(Pa, Pb)
