@@ -234,6 +234,26 @@ int rslam_map_initialize_features(rslam_filter* f, int b, int step, int min_feat
 /* Map::map_management (src/Map.cpp:16-67), all four steps; batch-1 handles only.  info4 = {deleted, converted index or -1,
  * initialised, attempts}. */
 int rslam_map_management(rslam_filter* f, int b, int step, int min_features, int reference_indexing, const double* u01, int n_pairs, int* info4);
+/* Map::map_management (src/Map.cpp:16-67), all four steps, for EVERY filter of the handle at once, each exactly as
+ * rslam_map_management does it on a batch-1 handle, in a fixed sequence of three kernel launches and one host synchronisation
+ * whatever the batch size and the number of edits.  Each filter's covariance is rewritten once (16 n^2 bytes), for all its
+ * deletions, its conversion and its new features together.
+ * u01: batch x (2 * n_pairs) uniforms (host or device); filter b's pairs start at u01 + 2 * n_pairs * b.  n_pairs >= 50.
+ * status[batch] (host): RSLAM_OK, RSLAM_ERR_REFERENCE_UB or RSLAM_ERR_CAPACITY per filter (RSLAM_ERR_INVALID: see below).
+ * info4[4 * batch] (host, optional): {deleted, converted index or -1, initialised, attempts} per filter.
+ * Returns RSLAM_OK, or the first non-OK per-filter status.
+ * Unlike rslam_map_management: a filter whose delete pass is undefined in the reference (RSLAM_ERR_REFERENCE_UB) is left exactly
+ * as it was (state, records, counters, flags) with info {deleted before the failure, -1, 0, 0}, and the other filters proceed; a
+ * filter that reaches max_features keeps the features added before, like the per-filter path (RSLAM_ERR_CAPACITY); n_pairs < 50,
+ * a NULL u01 or status, or a filter without a bound image return RSLAM_ERR_INVALID before any work.  One filter status can also be
+ * RSLAM_ERR_INVALID after work: an initialisation window that leaves the filter's image (uniforms outside [0, 1), or an image smaller
+ * than the camera) stops that filter's attempts, and like the per-filter path it keeps the edits made before (deletions, conversion,
+ * features already added).
+ * Memory: the first call allocates a spare covariance and state vector per filter (batch x ldp x (13 + 6 max_features) doubles
+ * more, ldp = that dimension rounded up to 16) and per-filter plans; the filters' buffers and the spares swap on each edit, so
+ * per-filter and batched calls can be mixed on one handle. */
+int rslam_map_management_batch(rslam_filter* f, int step, int min_features, int reference_indexing, const double* u01, int n_pairs, int* status,
+                               int* info4);
 
 #ifdef __cplusplus
 }

@@ -109,6 +109,7 @@ def load():
     L.rslam_fast_corner_detect_9.argtypes = [vp, ci, ci, ci, ci, ci, ci, ci, vp, vp]
     L.rslam_map_initialize_features.argtypes = [vp, ci, ci, ci, vp, ci, vp, vp]
     L.rslam_map_management.argtypes = [vp, ci, ci, ci, ci, vp, ci, vp]
+    L.rslam_map_management_batch.argtypes = [vp, ci, ci, ci, vp, ci, vp, vp]
     L.rslam_feature_types.argtypes = [vp, ci, vp]
     L.rslam_set_counters.argtypes = [vp, ci, vp, vp]
     L.rslam_download_feature_init.argtypes = [vp, ci, ci, vp, vp]
@@ -360,6 +361,22 @@ class Filter:
         if rc not in (0, -4):
             self._ck(rc)
         return rc, dict(deleted=int(info[0]), converted=int(info[1]), initialised=int(info[2]), attempts=int(info[3]))
+
+    def map_management_batch(self, step, min_features, u01, reference_indexing=True):
+        """Map::map_management for every filter at once.  u01: float64 [batch, 2 * n_pairs] on the host (n_pairs >= 50), or
+        (device ptr, n_pairs).  Returns (rc, status[batch], info[batch, 4]) with info rows (deleted, converted index or -1,
+        initialised, attempts); rc is 0 or the first non-zero status."""
+        if isinstance(u01, tuple):
+            up, n_pairs = C.c_void_p(u01[0]), int(u01[1])
+        else:
+            u = np.ascontiguousarray(u01, dtype=np.float64).reshape(self.batch, -1)
+            up, n_pairs = _p(u), u.shape[1] // 2
+        status = np.zeros(self.batch, dtype=np.int32)
+        info = np.zeros((self.batch, 4), dtype=np.int32)
+        rc = self.L.rslam_map_management_batch(self.h, int(step), int(min_features), int(reference_indexing), up, n_pairs, _p(status), _p(info))
+        if rc not in (0, -3, -4):
+            self._ck(rc)
+        return rc, status, info
 
     def types(self, b=0):
         N = self.L.rslam_num_features(self.h, b)

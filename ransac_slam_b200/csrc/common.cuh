@@ -98,7 +98,8 @@ enum CtlSlot {
     CTL_SIZE = 16
 };
 
-__device__ __forceinline__ void q2r_dev(const double* q, double R[9]) {  // src/ExtendKF.cpp:91-102
+// src/ExtendKF.cpp:91-102 (map_prep_add_dev in kernels_map.cuh has an unfused copy, kept in step by hand: change both)
+__device__ __forceinline__ void q2r_dev(const double* q, double R[9]) {
     const double r = q[0], x = q[1], y = q[2], z = q[3];
     R[0] = r * r + x * x - y * y - z * z;
     R[1] = 2 * (x * y - r * z);
@@ -239,7 +240,7 @@ __device__ __forceinline__ void distort_fixpoint_dev(const CamDev& cam, double u
     vd = yu / D / cam.dy + cam.Cy;
 }
 
-// Jacobian of the undistortion (src/ExtendKF.cpp:312-332), row-major 2x2
+// Jacobian of the undistortion (src/ExtendKF.cpp:312-332), row-major 2x2 (map_prep_add_dev in kernels_map.cuh has an unfused copy, kept in step by hand: change both)
 __device__ __forceinline__ void jacob_undistort_dev(const CamDev& cam, double ud, double vd, double J[4]) {
     const double a = ud - cam.Cx, b = vd - cam.Cy;
     const double adx = a * cam.dx, bdy = b * cam.dy;
@@ -252,7 +253,7 @@ __device__ __forceinline__ void jacob_undistort_dev(const CamDev& cam, double ud
     J[3] = c + b * g * (2 * b * cam.dy * cam.dy);
 }
 
-// d(R(q) a)/dq, 3x4 row-major (src/ExtendKF.cpp:286-311)
+// d(R(q) a)/dq, 3x4 row-major (src/ExtendKF.cpp:286-311) (map_prep_add_dev in kernels_map.cuh has an unfused copy, kept in step by hand: change both)
 __device__ __forceinline__ void dRq_times_a_by_dq_dev(const double* q, const double* a, double o[12]) {
     const double q0 = q[0], q1 = q[1], q2 = q[2], q3 = q[3];
     // column 0

@@ -8,16 +8,23 @@ namespace rslam {
 // ---------------------------------------------------------------------------------------------------------------
 // Map::map_management step 2 (src/Map.cpp:34-55): counters + per-frame flag reset.  One thread per feature.
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void k_begin_frame(DevFilter* Fs) {
-    DevFilter& F = Fs[blockIdx.y];
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= F.N) return;
+// for feature i; returns whether it was measured (li or hi) in the last frame
+__device__ __forceinline__ bool begin_frame_dev(const DevFilter& F, int i) {
+    const bool measured = F.li[i] || F.hi[i];
     if (F.has_h[i]) F.times_predicted[i] += 1;
-    if (F.li[i] || F.hi[i]) F.times_measured[i] += 1;
+    if (measured) F.times_measured[i] += 1;
     F.ic[i] = 0;
     F.li[i] = 0;
     F.hi[i] = 0;
     F.has_h[i] = 0;
+    return measured;
+}
+
+__global__ void k_begin_frame(DevFilter* Fs) {
+    DevFilter& F = Fs[blockIdx.y];
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= F.N) return;
+    begin_frame_dev(F, i);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -52,6 +52,16 @@ struct rslam_filter {
     double* map_coef = nullptr;
     int* map_res = nullptr;
     unsigned char* map_tmp = nullptr;  // staging for erasing one entry of the per-feature arrays
+    // rslam_map_management_batch (allocated on its first call): a spare covariance / state vector PER FILTER (B x ldp x nmax
+    // doubles more), swapped with the filter's own on every edit; per-filter plans and coefficients; pinned staging of its inputs
+    // (spare pointers, uniforms) and of its one read-back (plans)
+    std::vector<double*> mb_P, mb_x;
+    MapBatchWs mb{};
+    bool mb_ready = false;
+    void* mb_h_in = nullptr;   // pinned: [2B] spare pointers, then the uniforms
+    void* mb_d_in = nullptr;   // device copy of it
+    size_t mb_in_cap = 0;
+    int* mb_h_plan = nullptr;  // pinned: [B][MB_INTS] plans, then [B][Nmax] feature types
     int* fast_score = nullptr;         // FAST scores of the window under test
     size_t fast_cap = 0;
     int* fast_xy = nullptr;
@@ -548,6 +558,9 @@ int rslam_destroy(rslam_filter* f) {
     if (f->ev_free_cur) cudaEventDestroy(f->ev_free_cur);
     if (f->ev_free_pf) cudaEventDestroy(f->ev_free_pf);
     if (f->copy) cudaStreamDestroy(f->copy);
+    if (f->mb_h_in) cudaFreeHost(f->mb_h_in);
+    if (f->mb_d_in) cudaFree(f->mb_d_in);
+    if (f->mb_h_plan) cudaFreeHost(f->mb_h_plan);
     if (f->d_hyp_idx) cudaFree(f->d_hyp_idx);
     if (f->d_sup_h) cudaFree(f->d_sup_h);
     if (f->ev_fork) cudaEventDestroy(f->ev_fork);
@@ -1732,6 +1745,128 @@ int rslam_map_management(rslam_filter* f, int b, int step, int min_features, int
         info4[3] = attempts;
     }
     return rc;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Map::map_management for every filter of the handle in one fixed launch sequence (kernels_map.cuh, k_mmb_*)
+// ---------------------------------------------------------------------------------------------------------------------
+namespace {
+int ensure_map_batch_ws(rslam_filter* f) {
+    if (f->mb_ready) return 0;
+    const int B = f->B, Nmax = f->Nmax, nmax = f->nmax;
+    const int max_add = Nmax < kMbMaxAttempts ? Nmax : kMbMaxAttempts;
+    MapBatchWs& w = f->mb;
+    w.Nmax = Nmax;
+    w.nmax = nmax;
+    w.coef_stride = kMbAdd + max_add * kMbAddStride;
+    int rc;
+    double *P = nullptr, *x = nullptr;
+    if ((rc = dev_alloc(f, &P, (size_t)f->ldp * nmax * B, false))) return rc;
+    if ((rc = dev_alloc(f, &x, (size_t)nmax * B))) return rc;
+    if ((rc = dev_alloc(f, &w.plan, (size_t)MB_INTS * B))) return rc;
+    if ((rc = dev_alloc(f, &w.rowmap, (size_t)nmax * B))) return rc;
+    if ((rc = dev_alloc(f, &w.recsrc, (size_t)Nmax * B))) return rc;
+    if ((rc = dev_alloc(f, &w.rectail, (size_t)Nmax * B))) return rc;
+    if ((rc = dev_alloc(f, &w.types, (size_t)Nmax * B))) return rc;
+    if ((rc = dev_alloc(f, &w.vis, (size_t)Nmax * B))) return rc;
+    if ((rc = dev_alloc(f, &w.pix, (size_t)2 * Nmax * B))) return rc;
+    if ((rc = dev_alloc(f, &w.coef, (size_t)w.coef_stride * B))) return rc;
+    CK(cudaMallocHost((void**)&f->mb_h_plan, sizeof(int) * ((size_t)MB_INTS + Nmax) * B));
+    f->mb_P.resize(B);
+    f->mb_x.resize(B);
+    for (int b = 0; b < B; b++) {
+        f->mb_P[b] = P + (size_t)f->ldp * nmax * b;
+        f->mb_x[b] = x + (size_t)nmax * b;
+    }
+    f->mb_ready = true;
+    return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int rslam_map_management_batch(rslam_filter* f, int step, int min_features, int reference_indexing, const double* u01, int n_pairs, int* status,
+                               int* info4) {
+    (void)step;
+    if (!f || !u01 || !status || n_pairs < kMbMaxAttempts) return fail(RSLAM_ERR_INVALID, "rslam_map_management_batch: bad arguments (u01 and status are required, n_pairs >= %d)", kMbMaxAttempts);
+    for (int b = 0; b < f->B; b++)
+        if (!f->hF[b].image) return fail(RSLAM_ERR_INVALID, "rslam_map_management_batch: no image is bound to filter %d (rslam_set_image)", b);
+    CK(cudaSetDevice(f->device));
+    int rc;
+    if ((rc = ensure_map_batch_ws(f))) return rc;
+    const int B = f->B;
+    // inputs: the spare pointers and, from the host, the uniforms, in one copy from pinned staging
+    const bool u_dev = is_device_ptr(u01);
+    const size_t ptr_bytes = sizeof(double*) * 2 * B, u_bytes = u_dev ? 0 : sizeof(double) * 2 * n_pairs * B;
+    if (ptr_bytes + u_bytes > f->mb_in_cap) {
+        if (f->mb_h_in) CK(cudaFreeHost(f->mb_h_in));
+        if (f->mb_d_in) CK(cudaFree(f->mb_d_in));
+        f->mb_h_in = f->mb_d_in = nullptr;
+        f->mb_in_cap = 0;
+        CK(cudaMallocHost(&f->mb_h_in, ptr_bytes + u_bytes));
+        CK(cudaMalloc(&f->mb_d_in, ptr_bytes + u_bytes));
+        f->mb_in_cap = ptr_bytes + u_bytes;
+    }
+    double** hp = (double**)f->mb_h_in;
+    for (int b = 0; b < B; b++) {
+        hp[b] = f->mb_P[b];
+        hp[B + b] = f->mb_x[b];
+    }
+    if (!u_dev) memcpy((char*)f->mb_h_in + ptr_bytes, u01, u_bytes);
+    CK(cudaMemcpyAsync(f->mb_d_in, f->mb_h_in, ptr_bytes + u_bytes, cudaMemcpyHostToDevice, f->stream));
+    if (f->descr_dirty && (rc = push_descr(f))) return rc;
+    MapBatchWs w = f->mb;
+    w.Pdst = (double* const*)f->mb_d_in;
+    w.xdst = (double* const*)f->mb_d_in + B;
+    w.u01 = u_dev ? u01 : (const double*)((char*)f->mb_d_in + ptr_bytes);
+    w.n_pairs = n_pairs;
+    const int words = cdiv(f->nmax, 32);
+    const int max_add = f->Nmax < kMbMaxAttempts ? f->Nmax : kMbMaxAttempts;
+    const int nb = f->hn + 6 * max_add < f->nmax ? f->hn + 6 * max_add : f->nmax;  // bound on every filter's new state dimension
+    LAUNCH(f, k_mmb_plan, B, 256, sizeof(unsigned) * 2 * words, f->dF, w, min_features, reference_indexing);
+    // initial_rho = 1, std_rho = 1, std_pxl = std_z (src/Map.cpp:216-219), like rslam_map_add_feature
+    LAUNCH(f, k_mmb_init, B, 128, 0, f->dF, w, f->camd, 1.0, f->par.std_z, 1.0);
+    LAUNCH(f, k_mmb_xform, dim3(cdiv(nb, 256), cdiv(nb, kMbCols), B), 256, 0, f->dF, w);
+    if ((rc = check_launch())) return rc;
+    // the one read-back: per-filter plans and feature types
+    int* hplan = f->mb_h_plan;
+    int* htypes = hplan + (size_t)MB_INTS * B;
+    CK(cudaMemcpyAsync(hplan, w.plan, sizeof(int) * MB_INTS * B, cudaMemcpyDeviceToHost, f->stream));
+    CK(cudaMemcpyAsync(htypes, f->hF[0].ftype, sizeof(int) * (size_t)f->Nmax * B, cudaMemcpyDeviceToHost, f->stream));
+    CK(cudaStreamSynchronize(f->stream));
+    int first_bad_b = -1;
+    for (int b = 0; b < B; b++) {
+        const int* pl = hplan + (size_t)MB_INTS * b;
+        DevFilter& D = f->hF[b];
+        status[b] = pl[MB_STATUS];
+        if (info4) {
+            info4[4 * b] = pl[MB_DELETED];
+            info4[4 * b + 1] = pl[MB_CONVERTED];
+            info4[4 * b + 2] = pl[MB_INIT];
+            info4[4 * b + 3] = pl[MB_ATTEMPTS];
+        }
+        if (pl[MB_STATUS] != RSLAM_OK && first_bad_b < 0) first_bad_b = b;
+        if (pl[MB_STATUS] == RSLAM_ERR_REFERENCE_UB) continue;
+        if (pl[MB_EDIT]) {
+            std::swap(D.P, f->mb_P[b]);
+            std::swap(D.x_kk, f->mb_x[b]);
+        }
+        D.N = pl[MB_N];
+        D.n = pl[MB_NS];
+        const int* t = htypes + (size_t)f->Nmax * b;
+        f->htype[b].assign(t, t + D.N);
+    }
+    f->hN = 0;
+    f->hn = 0;
+    for (int k = 0; k < B; k++) {
+        f->hN = f->hF[k].N > f->hN ? f->hF[k].N : f->hN;
+        f->hn = f->hF[k].n > f->hn ? f->hF[k].n : f->hn;
+    }
+    if ((rc = push_descr(f))) return rc;
+    if (first_bad_b < 0) return RSLAM_OK;
+    return fail(status[first_bad_b], "rslam_map_management_batch: filter %d (the first of those that failed) returned %d", first_bad_b, status[first_bad_b]);
 }
 
 }  // extern "C"
