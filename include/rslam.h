@@ -255,6 +255,45 @@ int rslam_map_management(rslam_filter* f, int b, int step, int min_features, int
 int rslam_map_management_batch(rslam_filter* f, int step, int min_features, int reference_indexing, const double* u01, int n_pairs, int* status,
                                int* info4);
 
+/* --- checkpoint / resume of whole filters (not in the reference; SURVEY.md section 5) ---------------------------------------------
+ * A snapshot holds everything a filter carries from one frame to the next: n, N, the feature types, x_k_k, x_k_km1, the lower
+ * triangle of P and, per feature, times_predicted / times_measured, has_h / ic / li / hi, h, S, z, Hc, Hf, the predicted patch,
+ * patch_init and init_pose.  Loading it into a slot makes that slot continue exactly as the saved filter would have.  Not saved:
+ * the per-frame scratch (RANSAC and update workspaces, warp geometry; rslam_ransac_result_get of a loaded slot reads zeros until its
+ * next frame), the slot's image and uniform bindings (a loaded slot keeps its own), and handle-level switches (patch warp, graph).
+ * Both calls return when the copy is complete.  Host snapshots go through one device staging buffer of at most 256 MB, allocated by
+ * the first host-memory call and freed by rslam_destroy; device snapshots (memory on the handle's GPU, 16-byte aligned) are packed
+ * into and unpacked from directly.  Each chunk of at most 256 MB (one filter's records, or whole 64-column tile columns of its
+ * triangle) costs at most two kernel launches and one copy, whatever the batch size.
+ *
+ * Format, version 1: little-endian; every offset is from the start of the snapshot and every array starts 16-byte aligned;
+ * padding bytes are zero, so two saves of the same state are byte-for-byte equal.
+ *   header (160 bytes): char magic[8] = "RSLAMCKP"; u32 version = 1 (8); u32 count (12); u64 total bytes (16);
+ *     rslam_camera at 24: f64 k1, f64 k2, i32 nRows (40), i32 nCols (44), f64 Cx (48), Cy, f, dx, dy (up to 88);
+ *     rslam_params at 88: f64 std_a, std_alpha, std_z, chi2_095_2, corr_threshold, p_spurious_free (up to 136), i32 n_hyp_initial
+ *     (136), 4 zero bytes, f64 max_ellipse_eig (144), u32 quirks (152), i32 dedupe_hypotheses (156)
+ *   filter table at 160, count entries of 32 bytes: u64 block offset, u64 types offset, i32 n, i32 N, 8 zero bytes
+ *   feature types: i32[N] per filter, in filter order
+ *   filter blocks, in filter order: i32 n, i32 N, 8 zero bytes; then f64 x_k_k[n], f64 x_k_km1[n], i32 times_predicted[N],
+ *     i32 times_measured[N], u8 has_h[N], u8 ic[N], u8 li[N], u8 hi[N], f64 h[2N], f64 S[4N] (2 x 2 row-major), f64 z[2N],
+ *     f64 Hc[14N], f64 Hf[12N] (as rslam_download_H), f32 patch[169N] (13 x 13 row-major), u8 patch_init[1681N] (41 x 41 row-major),
+ *     f64 init_pose[14N] (r_wc, R_wc row-major, uv); then P as f64[n (n + 1) / 2] in LAPACK lower packed storage (UPLO = 'L':
+ *     column j holds rows j..n-1, so element (i, j), i >= j, is at j n - j (j - 1) / 2 + i - j). */
+/* size in bytes of a snapshot of filters [b, b + count) */
+int rslam_checkpoint_bytes(rslam_filter* f, int b, int count, size_t* bytes);
+/* snapshot of filters [b, b + count) into dst (host, or device memory on the handle's GPU).  cap too small: RSLAM_ERR_INVALID
+ * with the needed size in the message.  Every saved P must be exactly symmetric (bitwise, the library's invariant, checked on the
+ * device): otherwise RSLAM_ERR_INVALID naming the first filter that is not.  *written (optional) = the snapshot's size. */
+int rslam_checkpoint_save(rslam_filter* f, int b, int count, void* dst, size_t cap, size_t* written);
+/* restore every filter of the snapshot src[bytes] (host or device) into slots [b, b + count); *count_out (optional) = count.
+ * The handle may be another one, on this or another GPU, with any batch and any max_features >= each filter's N; its camera and
+ * params must equal the snapshot's bit for bit.  feature offsets and the last inverse-depth index are rebuilt from the types as
+ * rslam_upload_state builds them; each slot's x_k_k / x_k_km1 past the loaded n and its per-feature arrays past the loaded N are
+ * cleared, while its P outside the loaded n x n block is left as it was (as rslam_upload_state leaves it: no kernel reads P past n).  Refusals, all before any device
+ * write (the handle is unchanged): RSLAM_ERR_INVALID for a bad magic or version, a size other than the header's, an inconsistent
+ * table or types, a camera or params mismatch, or slots outside the batch; RSLAM_ERR_CAPACITY for N > max_features. */
+int rslam_checkpoint_load(rslam_filter* f, int b, const void* src, size_t bytes, int* count_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -44,6 +44,7 @@ EXPORTS = [
     "rslam_frame", "rslam_prefetch_inputs", "rslam_set_graph", "rslam_profile_enable", "rslam_profile_read", "rslam_download_pose", "rslam_support_sweep", "rslam_sweep_mask",
     "rslam_comm_init", "rslam_comm_unique_id", "rslam_comm_init_rank", "rslam_comm_destroy", "rslam_comm_size", "rslam_comm_local_size",
     "rslam_support_sweep_multi", "rslam_upload_linearisation", "rslam_predict_measurements", "rslam_match",
+    "rslam_checkpoint_bytes", "rslam_checkpoint_save", "rslam_checkpoint_load",
 ]
 
 _lib = None
@@ -113,6 +114,9 @@ def load():
     L.rslam_feature_types.argtypes = [vp, ci, vp]
     L.rslam_set_counters.argtypes = [vp, ci, vp, vp]
     L.rslam_download_feature_init.argtypes = [vp, ci, ci, vp, vp]
+    L.rslam_checkpoint_bytes.argtypes = [vp, ci, ci, C.POINTER(C.c_size_t)]
+    L.rslam_checkpoint_save.argtypes = [vp, ci, ci, vp, C.c_size_t, C.POINTER(C.c_size_t)]
+    L.rslam_checkpoint_load.argtypes = [vp, ci, vp, C.c_size_t, C.POINTER(ci)]
     _lib = L
     return L
 
@@ -396,6 +400,41 @@ class Filter:
         self._ck(self.L.rslam_download_feature_init(self.h, b, int(i), _p(patch), _p(pose)))
         return patch, pose
 
+    # ---- checkpoint / resume (format: include/rslam.h; read_checkpoint below parses it without a GPU) ----
+    def checkpoint_bytes(self, b=0, count=None):
+        count = self.batch - b if count is None else count
+        nb = C.c_size_t(0)
+        self._ck(self.L.rslam_checkpoint_bytes(self.h, b, count, C.byref(nb)))
+        return nb.value
+
+    def save(self, b=0, count=None, out=None):
+        """snapshot of filters [b, b + count) (default: to the end of the batch).  out: None (a new np.uint8 array), a host np.uint8
+        array, or a CUDA uint8 tensor on the handle's GPU (saved without host staging).  Returns out[:size] (or the new array)."""
+        count = self.batch - b if count is None else count
+        if out is None:
+            out = np.empty(self.checkpoint_bytes(b, count), dtype=np.uint8)
+        written = C.c_size_t(0)
+        if isinstance(out, np.ndarray):
+            assert out.dtype == np.uint8 and out.flags.c_contiguous
+            ptr, cap = _p(out), out.size
+        else:  # torch tensor
+            assert out.dtype.itemsize == 1 and out.is_contiguous()
+            ptr, cap = C.c_void_p(out.data_ptr()), out.numel()
+        self._ck(self.L.rslam_checkpoint_save(self.h, b, count, ptr, cap, C.byref(written)))
+        return out[: written.value]
+
+    def load(self, buf, b=0):
+        """restore every filter of the snapshot buf (np.uint8 array or CUDA uint8 tensor) into slots b, b + 1, ...; returns the count"""
+        if isinstance(buf, np.ndarray):
+            buf = np.ascontiguousarray(buf, dtype=np.uint8)
+            ptr, nb = _p(buf), buf.size
+        else:
+            assert buf.dtype.itemsize == 1 and buf.is_contiguous()
+            ptr, nb = C.c_void_p(buf.data_ptr()), buf.numel()
+        cnt = C.c_int(0)
+        self._ck(self.L.rslam_checkpoint_load(self.h, b, ptr, nb, C.byref(cnt)))
+        return cnt.value
+
     def set_graph(self, enable):
         self._ck(self.L.rslam_set_graph(self.h, int(enable)))
 
@@ -454,6 +493,66 @@ class Filter:
         mask = np.zeros((self.max_features + 7) // 8, dtype=np.uint8)
         self._ck(self.L.rslam_sweep_mask(self.h, int(match_idx), _p(mask)))
         return np.unpackbits(mask, bitorder="little").astype(bool)
+
+
+CHECKPOINT_MAGIC = b"RSLAMCKP"
+CHECKPOINT_VERSION = 1
+_CK_CAMERA = [("k1", "<f8", 24), ("k2", "<f8", 32), ("nRows", "<i4", 40), ("nCols", "<i4", 44), ("Cx", "<f8", 48), ("Cy", "<f8", 56),
+              ("f", "<f8", 64), ("dx", "<f8", 72), ("dy", "<f8", 80)]
+_CK_PARAMS = [("std_a", "<f8", 88), ("std_alpha", "<f8", 96), ("std_z", "<f8", 104), ("chi2_095_2", "<f8", 112), ("corr_threshold", "<f8", 120),
+              ("p_spurious_free", "<f8", 128), ("n_hyp_initial", "<i4", 136), ("max_ellipse_eig", "<f8", 144), ("quirks", "<u4", 152),
+              ("dedupe_hypotheses", "<i4", 156)]
+# per-filter record arrays after the 16-byte head, in order: (name, dtype, shape per unit, unit "n" or "N")
+_CK_RECORDS = [("x", "<f8", (), "n"), ("x_k_km1", "<f8", (), "n"), ("times_predicted", "<i4", (), "N"), ("times_measured", "<i4", (), "N"),
+               ("has_h", "u1", (), "N"), ("ic", "u1", (), "N"), ("li", "u1", (), "N"), ("hi", "u1", (), "N"), ("h", "<f8", (2,), "N"),
+               ("S", "<f8", (2, 2), "N"), ("z", "<f8", (2,), "N"), ("Hc", "<f8", (2, 7), "N"), ("Hf", "<f8", (2, 6), "N"),
+               ("patches", "<f4", (13, 13), "N"), ("patch41", "u1", (41, 41), "N"), ("pose14", "<f8", (14,), "N")]
+
+
+def _al16(v):
+    return (v + 15) & ~15
+
+
+def read_checkpoint(buf):
+    """Parse a snapshot of rslam_checkpoint_save (pure numpy, no GPU).  Returns (header, filters): header = dict(version, count,
+    camera=dict, params=dict); filters = list of dicts with n, N, types and the record arrays (x, x_k_km1, counters, flags, h, S, z,
+    Hc, Hf, patches, patch41, pose14), and P expanded from the packed lower triangle to the full square."""
+    buf = np.frombuffer(bytes(buf) if not isinstance(buf, np.ndarray) else np.ascontiguousarray(buf, dtype=np.uint8).tobytes(), dtype=np.uint8)
+
+    def at(dt, off, count=1):
+        return np.frombuffer(buf, dtype=np.dtype(dt), count=count, offset=off)
+
+    if buf.size < 160 or buf[:8].tobytes() != CHECKPOINT_MAGIC:
+        raise ValueError("not an rslam snapshot (bad magic)")
+    version, count = int(at("<u4", 8)[0]), int(at("<u4", 12)[0])
+    total = int(at("<u8", 16)[0])
+    if version != CHECKPOINT_VERSION or total != buf.size:
+        raise ValueError(f"snapshot version {version}, {total} bytes declared, {buf.size} given")
+    header = dict(version=version, count=count, camera={k: at(d, o)[0].item() for k, d, o in _CK_CAMERA},
+                  params={k: at(d, o)[0].item() for k, d, o in _CK_PARAMS})
+    filters = []
+    for i in range(count):
+        e = 160 + 32 * i
+        boff, toff = int(at("<u8", e)[0]), int(at("<u8", e + 8)[0])
+        n, N = int(at("<i4", e + 16)[0]), int(at("<i4", e + 20)[0])
+        hn, hN = at("<i4", boff, 2)
+        assert (hn, hN) == (n, N), (i, hn, hN, n, N)
+        d = dict(n=n, N=N, types=at("<i4", toff, N).copy())
+        o = boff + 16
+        for name, dt, shape, unit in _CK_RECORDS:
+            cnt = (n if unit == "n" else N) * int(np.prod(shape, dtype=np.int64))
+            d[name] = at(dt, o, cnt).reshape(((n,) if unit == "n" else (N,) + shape)).copy()
+            o += _al16(cnt * np.dtype(dt).itemsize)
+        for name in ("has_h", "ic", "li", "hi"):
+            d[name] = d[name].astype(bool)
+        packed = at("<f8", o, n * (n + 1) // 2)
+        P = np.zeros((n, n), order="F")
+        j, i = np.triu_indices(n)  # (j, i), i >= j, in row-major order: column j of the lower triangle, rows j..n-1 (LAPACK 'L')
+        P[i, j] = packed
+        P[j, i] = packed
+        d["P"] = P
+        filters.append(d)
+    return header, filters
 
 
 def decode_key(key):

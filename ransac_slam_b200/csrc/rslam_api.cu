@@ -9,6 +9,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "kernels_ckpt.cuh"
 #include "kernels_map.cuh"
 #include "kernels_track.cuh"
 #include "kernels_update.cuh"
@@ -62,6 +63,12 @@ struct rslam_filter {
     void* mb_d_in = nullptr;   // device copy of it
     size_t mb_in_cap = 0;
     int* mb_h_plan = nullptr;  // pinned: [B][MB_INTS] plans, then [B][Nmax] feature types
+    // rslam_checkpoint_save / _load: the device staging buffer of host-memory snapshots (<= 256 MB, allocated by the first such
+    // call) and the work lists of the current call (chunk records and tiles, then the per-filter symmetry flags)
+    unsigned char* ck_stage = nullptr;
+    size_t ck_stage_cap = 0;
+    unsigned char* ck_list = nullptr;
+    size_t ck_list_cap = 0;
     int* fast_score = nullptr;         // FAST scores of the window under test
     size_t fast_cap = 0;
     int* fast_xy = nullptr;
@@ -561,6 +568,8 @@ int rslam_destroy(rslam_filter* f) {
     if (f->mb_h_in) cudaFreeHost(f->mb_h_in);
     if (f->mb_d_in) cudaFree(f->mb_d_in);
     if (f->mb_h_plan) cudaFreeHost(f->mb_h_plan);
+    if (f->ck_stage) cudaFree(f->ck_stage);
+    if (f->ck_list) cudaFree(f->ck_list);
     if (f->d_hyp_idx) cudaFree(f->d_hyp_idx);
     if (f->d_sup_h) cudaFree(f->d_sup_h);
     if (f->ev_fork) cudaEventDestroy(f->ev_fork);
@@ -1867,6 +1876,346 @@ int rslam_map_management_batch(rslam_filter* f, int step, int min_features, int 
     if ((rc = push_descr(f))) return rc;
     if (first_bad_b < 0) return RSLAM_OK;
     return fail(status[first_bad_b], "rslam_map_management_batch: filter %d (the first of those that failed) returned %d", first_bad_b, status[first_bad_b]);
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Checkpoint / resume of whole filters (kernels_ckpt.cuh; the snapshot format is documented in include/rslam.h)
+// ---------------------------------------------------------------------------------------------------------------------
+namespace {
+constexpr size_t kCkHeader = 160, kCkEntry = 32, kCkStageMax = (size_t)256 << 20;
+constexpr uint32_t kCkVersion = 1;
+const char kCkMagic[8] = {'R', 'S', 'L', 'A', 'M', 'C', 'K', 'P'};
+
+// camera and params at their fixed offsets (bytes 24..159 of the header; the library only builds for little-endian hosts)
+void ck_put_config(const rslam_filter* f, unsigned char* h) {
+    auto pd = [h](size_t o, double v) { memcpy(h + o, &v, 8); };
+    auto pi = [h](size_t o, int32_t v) { memcpy(h + o, &v, 4); };
+    memset(h + 24, 0, kCkHeader - 24);
+    const rslam_camera& c = f->cam;
+    const rslam_params& p = f->par;
+    pd(24, c.k1), pd(32, c.k2), pi(40, c.nRows), pi(44, c.nCols), pd(48, c.Cx), pd(56, c.Cy), pd(64, c.f), pd(72, c.dx), pd(80, c.dy);
+    pd(88, p.std_a), pd(96, p.std_alpha), pd(104, p.std_z), pd(112, p.chi2_095_2), pd(120, p.corr_threshold), pd(128, p.p_spurious_free);
+    pi(136, p.n_hyp_initial), pd(144, p.max_ellipse_eig), pi(152, (int32_t)p.quirks), pi(156, p.dedupe_hypotheses);
+}
+
+// where everything of a snapshot of filters with these n / N lies
+struct CkLayout {
+    std::vector<int> n, N;
+    std::vector<size_t> types_off, block_off;
+    size_t dir_bytes = 0, total = 0;
+    void build() {
+        const size_t count = n.size();
+        types_off.resize(count);
+        block_off.resize(count);
+        size_t o = kCkHeader + kCkEntry * count;
+        for (size_t i = 0; i < count; i++) {
+            types_off[i] = o;
+            o += ck_al16(4 * (size_t)N[i]);
+        }
+        dir_bytes = o;
+        for (size_t i = 0; i < count; i++) {
+            block_off[i] = o;
+            o += ck_rec_bytes(n[i], N[i]) + ck_tri_bytes(n[i]);
+        }
+        total = o;
+    }
+};
+
+// header, filter table and feature types of filters [b, b + count) (from the host mirror)
+void ck_put_directory(const rslam_filter* f, const CkLayout& L, int b, unsigned char* h) {
+    memset(h, 0, L.dir_bytes);
+    memcpy(h, kCkMagic, 8);
+    const uint32_t ver = kCkVersion, cnt = (uint32_t)L.n.size();
+    const uint64_t tot = L.total;
+    memcpy(h + 8, &ver, 4);
+    memcpy(h + 12, &cnt, 4);
+    memcpy(h + 16, &tot, 8);
+    ck_put_config(f, h);
+    for (size_t i = 0; i < L.n.size(); i++) {
+        unsigned char* e = h + kCkHeader + kCkEntry * i;
+        const uint64_t bo = L.block_off[i], to = L.types_off[i];
+        memcpy(e, &bo, 8);
+        memcpy(e + 8, &to, 8);
+        memcpy(e + 16, &L.n[i], 4);
+        memcpy(e + 20, &L.N[i], 4);
+        if (L.N[i]) memcpy(h + L.types_off[i], f->htype[b + i].data(), 4 * (size_t)L.N[i]);
+    }
+}
+
+// Consecutive pieces of the stream of filter blocks, each at most `cap` bytes: a filter's records, or a range of whole 64-column
+// tile columns of its triangle; with the work items of each piece (records and lower tiles, offsets relative to the piece)
+struct CkChunk {
+    size_t off, bytes;
+    int rec0, nrec, tile0, ntile;
+};
+struct CkPlan {
+    std::vector<CkptRec> recs;
+    std::vector<CkptTile> tiles;
+    std::vector<CkChunk> chunks;
+    size_t max_chunk = 0;
+};
+int ck_plan(const CkLayout& L, int b, size_t cap, CkPlan& p) {
+    CkChunk cur{L.dir_bytes, 0, 0, 0, 0, 0};
+    auto close = [&](size_t start) {
+        if (cur.bytes) {
+            p.chunks.push_back(cur);
+            p.max_chunk = cur.bytes > p.max_chunk ? cur.bytes : p.max_chunk;
+        }
+        cur = CkChunk{start, 0, (int)p.recs.size(), 0, (int)p.tiles.size(), 0};
+    };
+    for (size_t i = 0; i < L.n.size(); i++) {
+        const long long n = L.n[i];
+        const size_t rb = ck_rec_bytes(n, L.N[i]), pstart = L.block_off[i] + rb;
+        if (rb > cap) return fail(RSLAM_ERR_CAPACITY, "checkpoint: the records of one filter (%zu bytes) exceed the %zu-byte staging buffer", rb, cap);
+        if (cur.bytes && pstart - cur.off > cap) close(L.block_off[i]);
+        p.recs.push_back(CkptRec{b + (int)i, (int)n, L.N[i], 0, (long long)(L.block_off[i] - cur.off)});
+        cur.nrec++;
+        cur.bytes = pstart - cur.off;
+        const int T = cdiv((int)n, kCkTile);
+        for (int J = 0; J < T; J++) {
+            const long long j0 = (long long)kCkTile * J, j1 = j0 + kCkTile < n ? j0 + kCkTile : n;
+            const size_t s = pstart + 8 * (size_t)ck_colstart(j0, n);
+            const size_t e = J == T - 1 ? pstart + ck_tri_bytes(n) : pstart + 8 * (size_t)ck_colstart(j1, n);
+            if (e - s > cap) return fail(RSLAM_ERR_CAPACITY, "checkpoint: one tile column (%zu bytes) exceeds the %zu-byte staging buffer", e - s, cap);
+            if (cur.bytes && e - cur.off > cap) close(s);  // s is 16-byte aligned: the column start of a 64-column boundary is even
+            const long long pbase = ((long long)pstart - (long long)cur.off) / 8;
+            for (int I = J; I < T; I++) p.tiles.push_back(CkptTile{b + (int)i, (int)n, I, J, pbase});
+            cur.ntile += T - J;
+            cur.bytes = e - cur.off;
+        }
+    }
+    close(0);
+    return 0;
+}
+
+// 1: device memory on the handle's GPU, 0: host memory, -1: device memory of another GPU
+int ck_where(const rslam_filter* f, const void* p) {
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+        cudaGetLastError();
+        return 0;
+    }
+    if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) return 0;
+    return at.device == f->device ? 1 : -1;
+}
+
+int ck_grow(rslam_filter* f, unsigned char** p, size_t* cap, size_t need) {
+    if (need <= *cap) return 0;
+    if (*p) {
+        CK(cudaStreamSynchronize(f->stream));
+        CK(cudaFree(*p));
+    }
+    *p = nullptr;
+    *cap = 0;
+    CK(cudaMalloc((void**)p, need));
+    *cap = need;
+    return 0;
+}
+
+// the work lists of a plan on the device, followed by `count` zeroed symmetry flags
+int ck_push_lists(rslam_filter* f, const CkPlan& p, int count, CkptRec** drec, CkptTile** dtile, int** dbad) {
+    const size_t rb = sizeof(CkptRec) * p.recs.size(), tb = sizeof(CkptTile) * p.tiles.size();
+    int rc = ck_grow(f, &f->ck_list, &f->ck_list_cap, rb + tb + sizeof(int) * count + 16);
+    if (rc) return rc;
+    std::vector<unsigned char> h(rb + tb);
+    if (rb) memcpy(h.data(), p.recs.data(), rb);
+    if (tb) memcpy(h.data() + rb, p.tiles.data(), tb);
+    // pageable source: staged before the call returns, so the vector may go
+    CK(cudaMemcpyAsync(f->ck_list, h.data(), rb + tb, cudaMemcpyHostToDevice, f->stream));
+    CK(cudaMemsetAsync(f->ck_list + rb + tb, 0, sizeof(int) * count, f->stream));
+    *drec = (CkptRec*)f->ck_list;
+    *dtile = (CkptTile*)(f->ck_list + rb);
+    *dbad = (int*)(f->ck_list + rb + tb);
+    return 0;
+}
+
+int ck_range(rslam_filter* f, int b, int count, CkLayout& L, const char* who) {
+    if (!f || b < 0 || count < 1 || count > f->B - b) return fail(RSLAM_ERR_INVALID, "%s: filters [%d, %d + %d) are not in the handle", who, b, b, count);
+    for (int i = 0; i < count; i++) {
+        L.n.push_back(f->hF[b + i].n);
+        L.N.push_back(f->hF[b + i].N);
+    }
+    L.build();
+    return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int rslam_checkpoint_bytes(rslam_filter* f, int b, int count, size_t* bytes) {
+    CkLayout L;
+    int rc = ck_range(f, b, count, L, "rslam_checkpoint_bytes");
+    if (rc) return rc;
+    if (!bytes) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_bytes: bytes is NULL");
+    *bytes = L.total;
+    return RSLAM_OK;
+}
+
+int rslam_checkpoint_save(rslam_filter* f, int b, int count, void* dst, size_t cap, size_t* written) {
+    CkLayout L;
+    int rc = ck_range(f, b, count, L, "rslam_checkpoint_save");
+    if (rc) return rc;
+    if (!dst) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_save: dst is NULL");
+    CK(cudaSetDevice(f->device));
+    const int where = ck_where(f, dst);
+    if (where < 0) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_save: dst is device memory of another GPU than the handle's (%d)", f->device);
+    if (where == 1 && ((uintptr_t)dst & 15)) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_save: device dst must be 16-byte aligned");
+    if (cap < L.total) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_save: cap = %zu bytes, the snapshot needs %zu", cap, L.total);
+    const bool dev = where == 1;
+    CkPlan p;
+    if ((rc = ck_plan(L, b, dev ? (size_t)-1 : kCkStageMax, p))) return rc;
+    if (!dev && (rc = ck_grow(f, &f->ck_stage, &f->ck_stage_cap, p.max_chunk))) return rc;
+    if (f->descr_dirty && (rc = push_descr(f))) return rc;
+    CkptRec* drec;
+    CkptTile* dtile;
+    int* dbad;
+    if ((rc = ck_push_lists(f, p, count, &drec, &dtile, &dbad))) return rc;
+    std::vector<unsigned char> dir(L.dir_bytes);
+    ck_put_directory(f, L, b, dir.data());
+    if (dev)
+        CK(cudaMemcpyAsync(dst, dir.data(), L.dir_bytes, cudaMemcpyHostToDevice, f->stream));
+    else
+        memcpy(dst, dir.data(), L.dir_bytes);
+    for (const CkChunk& c : p.chunks) {
+        unsigned char* base = dev ? (unsigned char*)dst + c.off : f->ck_stage;
+        if (c.nrec) LAUNCH(f, k_ckpt_records_pack, dim3(c.nrec, kCkSegs), 256, 0, f->dF, drec + c.rec0, base);
+        if (c.ntile) LAUNCH(f, k_ckpt_pack, c.ntile, 256, 0, f->dF, dtile + c.tile0, (double*)base, dbad, b);
+        if ((rc = check_launch())) return rc;
+        if (!dev) CK(cudaMemcpyAsync((unsigned char*)dst + c.off, f->ck_stage, c.bytes, cudaMemcpyDeviceToHost, f->stream));
+    }
+    std::vector<int> bad(count);
+    CK(cudaMemcpyAsync(bad.data(), dbad, sizeof(int) * count, cudaMemcpyDeviceToHost, f->stream));
+    CK(cudaStreamSynchronize(f->stream));
+    for (int i = 0; i < count; i++)
+        if (bad[i]) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_save: P of filter %d is not exactly symmetric (bitwise)", b + i);
+    if (written) *written = L.total;
+    return RSLAM_OK;
+}
+
+int rslam_checkpoint_load(rslam_filter* f, int b, const void* src, size_t bytes, int* count_out) {
+    if (!f || !src) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: bad arguments");
+    CK(cudaSetDevice(f->device));
+    const int where = ck_where(f, src);
+    if (where < 0) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: src is device memory of another GPU than the handle's (%d)", f->device);
+    if (where == 1 && ((uintptr_t)src & 15)) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: device src must be 16-byte aligned");
+    const bool dev = where == 1;
+    // everything is validated on the host before the first device write
+    auto fetch = [&](void* h, size_t off, size_t len) -> int {
+        if (!dev) {
+            memcpy(h, (const unsigned char*)src + off, len);
+            return 0;
+        }
+        CK(cudaMemcpyAsync(h, (const unsigned char*)src + off, len, cudaMemcpyDeviceToHost, f->stream));
+        CK(cudaStreamSynchronize(f->stream));
+        return 0;
+    };
+    int rc;
+    if (bytes < kCkHeader) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: %zu bytes is shorter than the header", bytes);
+    unsigned char hdr[kCkHeader], mine[kCkHeader];
+    if ((rc = fetch(hdr, 0, kCkHeader))) return rc;
+    if (memcmp(hdr, kCkMagic, 8)) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: not a snapshot (bad magic)");
+    uint32_t ver, cnt;
+    uint64_t tot;
+    memcpy(&ver, hdr + 8, 4);
+    memcpy(&cnt, hdr + 12, 4);
+    memcpy(&tot, hdr + 16, 8);
+    if (ver != kCkVersion) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: format version %u, this library reads %u", ver, kCkVersion);
+    if (tot != bytes) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: the snapshot is %llu bytes, the buffer %zu", (unsigned long long)tot, bytes);
+    ck_put_config(f, mine);
+    if (memcmp(hdr + 24, mine + 24, kCkHeader - 24)) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: camera or params differ from the handle's");
+    if (cnt < 1 || b < 0 || (long long)b + cnt > f->B) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: %u filters do not fit at slot %d of a batch of %d", cnt, b, f->B);
+    const int count = (int)cnt;
+    if (kCkHeader + kCkEntry * (size_t)count > bytes) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: truncated filter table");
+    std::vector<unsigned char> tab(kCkEntry * (size_t)count);
+    if ((rc = fetch(tab.data(), kCkHeader, tab.size()))) return rc;
+    CkLayout L;
+    for (int i = 0; i < count; i++) {
+        int n, N;
+        memcpy(&n, &tab[kCkEntry * i + 16], 4);
+        memcpy(&N, &tab[kCkEntry * i + 20], 4);
+        if (N < 0 || N > (1 << 24) || n < 13 + 3 * N || n > 13 + 6 * N) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: filter %d has n = %d, N = %d", i, n, N);
+        L.n.push_back(n);
+        L.N.push_back(N);
+    }
+    L.build();
+    if (L.total != bytes) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: the filter table describes %zu bytes, the buffer holds %zu", L.total, bytes);
+    for (int i = 0; i < count; i++) {
+        uint64_t bo, to;
+        memcpy(&bo, &tab[kCkEntry * i], 8);
+        memcpy(&to, &tab[kCkEntry * i + 8], 8);
+        if (bo != L.block_off[i] || to != L.types_off[i]) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: filter %d is not where the table says", i);
+    }
+    const size_t t0 = kCkHeader + kCkEntry * (size_t)count;
+    std::vector<unsigned char> traw(L.dir_bytes - t0);
+    if (!traw.empty() && (rc = fetch(traw.data(), t0, traw.size()))) return rc;
+    std::vector<std::vector<int>> types(count);
+    for (int i = 0; i < count; i++) {
+        types[i].resize(L.N[i]);
+        if (L.N[i]) memcpy(types[i].data(), traw.data() + (L.types_off[i] - t0), 4 * (size_t)L.N[i]);
+        int n = 13;
+        for (int t : types[i]) {
+            if (t != 0 && t != 1) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: filter %d has a feature type %d", i, t);
+            n += t == 0 ? 6 : 3;
+        }
+        if (n != L.n[i]) return fail(RSLAM_ERR_INVALID, "rslam_checkpoint_load: filter %d has n = %d, but 13 + sum(feature sizes) = %d", i, L.n[i], n);
+    }
+    for (int i = 0; i < count; i++)
+        if (L.N[i] > f->Nmax) return fail(RSLAM_ERR_CAPACITY, "rslam_checkpoint_load: filter %d has %d features > max_features %d", i, L.N[i], f->Nmax);
+    CkPlan p;
+    if ((rc = ck_plan(L, b, dev ? (size_t)-1 : kCkStageMax, p))) return rc;
+    if (!dev && (rc = ck_grow(f, &f->ck_stage, &f->ck_stage_cap, p.max_chunk))) return rc;
+    // device writes from here on
+    if (f->descr_dirty && (rc = push_descr(f))) return rc;
+    CkptRec* drec;
+    CkptTile* dtile;
+    int* dbad;
+    if ((rc = ck_push_lists(f, p, count, &drec, &dtile, &dbad))) return rc;
+    for (const CkChunk& c : p.chunks) {
+        const unsigned char* base = dev ? (const unsigned char*)src + c.off : f->ck_stage;
+        if (!dev) CK(cudaMemcpyAsync(f->ck_stage, (const unsigned char*)src + c.off, c.bytes, cudaMemcpyHostToDevice, f->stream));
+        if (c.nrec) LAUNCH(f, k_ckpt_records_unpack, dim3(c.nrec, kCkSegs - 1), 256, 0, f->dF, drec + c.rec0, base, f->nmax, f->Nmax);
+        if (c.ntile) LAUNCH(f, k_ckpt_unpack, c.ntile, 256, 0, f->dF, dtile + c.tile0, (const double*)base);
+        if ((rc = check_launch())) return rc;
+    }
+    // feature types, offsets and last inverse-depth index as rslam_upload_state builds them, cleared past N; the slots' arrays are
+    // consecutive pieces (stride max_features) of one allocation each, as are their RANSAC control blocks, cleared here
+    const size_t per = (size_t)f->Nmax;
+    std::vector<int> ht(per * count * 3, 0);
+    int* hty = ht.data();
+    int* hof = hty + per * count;
+    int* hli = hof + per * count;
+    for (int i = 0; i < count; i++)
+        for (int k = 0, off = 13, last = -1; k < L.N[i]; k++) {
+            const int t = types[i][k];
+            if (t == 0) last = k;
+            hty[per * i + k] = t;
+            hof[per * i + k] = off;
+            hli[per * i + k] = last;
+            off += t == 0 ? 6 : 3;
+        }
+    const DevFilter& D0 = f->hF[b];
+    CK(cudaMemcpyAsync(D0.ftype, hty, sizeof(int) * per * count, cudaMemcpyHostToDevice, f->stream));
+    CK(cudaMemcpyAsync(D0.foff, hof, sizeof(int) * per * count, cudaMemcpyHostToDevice, f->stream));
+    CK(cudaMemcpyAsync(D0.last_id, hli, sizeof(int) * per * count, cudaMemcpyHostToDevice, f->stream));
+    CK(cudaMemsetAsync(D0.ctl, 0, sizeof(int) * CTL_SIZE * count, f->stream));
+    CK(cudaStreamSynchronize(f->stream));
+    for (int i = 0; i < count; i++) {
+        DevFilter& D = f->hF[b + i];
+        D.n = L.n[i];
+        D.N = L.N[i];
+        f->htype[b + i] = types[i];
+    }
+    f->hN = 0;
+    f->hn = 0;
+    for (int k = 0; k < f->B; k++) {
+        f->hN = f->hF[k].N > f->hN ? f->hF[k].N : f->hN;
+        f->hn = f->hF[k].n > f->hn ? f->hF[k].n : f->hn;
+    }
+    if ((rc = push_descr(f))) return rc;
+    if (count_out) *count_out = count;
+    return RSLAM_OK;
 }
 
 }  // extern "C"
