@@ -59,7 +59,8 @@ typedef struct {
     double corr_threshold;          /* 0.80   (src/Tracking.cpp:281) */
     double p_spurious_free;         /* 0.99   (src/Tracking.cpp:354) */
     int n_hyp_initial;              /* 1000   (src/Tracking.cpp:357) */
-    double max_ellipse_eig;         /* 100    (src/Tracking.cpp:303) */
+    double max_ellipse_eig;         /* 100    (src/Tracking.cpp:303); rslam_create refuses a value that is not in (0, 100] (RSLAM_ERR_INVALID):
+                                       the active search stages windows of half-width ceil(2 sqrt(S_ii)) <= 20, which lmax < 100 guarantees */
     unsigned quirks;                /* RSLAM_Q_* mask, default RSLAM_Q_ALL */
     int dedupe_hypotheses;          /* 1: score each distinct 1-point hypothesis once (identical results) */
 } rslam_params;
@@ -112,7 +113,10 @@ int rslam_download_H(rslam_filter* f, int b, double* Hc, double* Hf);
 int rslam_upload_linearisation(rslam_filter* f, int b, const double* h, const double* Hc, const double* Hf, const double* z, const uint8_t* flags);
 /* inject matches directly (z[2N], ic[N]) instead of running the active search */
 int rslam_set_matches(rslam_filter* f, int b, const double* z, const uint8_t* ic);
-/* grayscale frame for filter b (host or device).  With share != 0 the same image is used by every filter of the batch. */
+/* grayscale frame for filter b (host or device).  With share != 0 the same image is used by every filter of the batch.
+ * Binding an image to one filter never changes what any other filter reads: a host image is copied into a device buffer owned by
+ * filter b (share == 0) or by the batch's shared image (share != 0), whatever the geometry of earlier calls; a device image is read
+ * in place and must stay valid while filters are bound to it. */
 int rslam_set_image(rslam_filter* f, int b, const uint8_t* gray, int rows, int cols, int stride, int share);
 
 /* --- the per-frame path (src/System.cpp:111-129) ------------------------------------------------------------- */

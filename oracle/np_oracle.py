@@ -108,6 +108,64 @@ def jacobian_H(cam, x, types, i, h_i):
     return H
 
 
+def v2q(v, eps=2.220446049250313e-16):  # src/ExtendKF.cpp:428-443 (quirk Q14: the zero quaternion below eps)
+    theta = np.sqrt(v @ v)
+    if theta < eps:
+        return np.zeros(4)
+    vn = v / theta
+    return np.concatenate([[np.cos(theta / 2.0)], np.sin(theta / 2.0) * (vn / np.sqrt(vn @ vn))])
+
+
+def qprod(q, p):  # src/ExtendKF.cpp:416-427: q * p with the vector part (q0 p_v + p0 q_v) + q_v x p_v
+    return np.concatenate([[q[0] * p[0] - q[1:] @ p[1:]], q[0] * p[1:] + p[0] * q[1:] + np.cross(q[1:], p[1:])])
+
+
+def dq3_by_dq1(q):  # src/ExtendKF.cpp:482-490
+    return np.array([[q[0], -q[1], -q[2], -q[3]], [q[1], q[0], -q[3], q[2]], [q[2], q[3], q[0], -q[1]], [q[3], -q[2], q[1], q[0]]])
+
+
+def dqomegadt_by_domega(w, dt=1.0):  # src/ExtendKF.cpp:491-529
+    om = np.sqrt(w @ w)
+    s, c = np.sin(om * dt / 2.0), np.cos(om * dt / 2.0)
+    m = np.zeros((4, 3))
+    m[0] = (-dt / 2.0) * (w / om) * s
+    for i in range(3):
+        for j in range(3):
+            if i == j:
+                m[1 + i, j] = (dt / 2.0) * w[i] * w[i] / (om * om) * c + (1.0 / om) * (1.0 - w[i] * w[i] / (om * om)) * s
+            else:
+                m[1 + i, j] = (w[i] * w[j] / (om * om)) * ((dt / 2.0) * c - (1.0 / om) * s)
+    return m
+
+
+def ekf_prediction(x, P, std_a, std_alpha, dt=1.0):
+    """ExtendKF::ekf_prediction (src/ExtendKF.cpp:333-388), constant velocity: x_k_km1 = [fv(x_v); y] and
+    P_k_km1 = [F P_cc F^T + Q, F P_cf; P_fc F^T, P_ff] with F = dfv_by_dxv (:444-481) and Q = G diag(la, la, la, aa, aa, aa) G^T
+    (:347-376).  Returns (x_k_km1, P_k_km1)."""
+    x = np.asarray(x, dtype=np.float64)
+    qwt = v2q(x[10:13] * dt)
+    xv = np.concatenate([x[0:3] + x[7:10] * dt, qprod(x[3:7], qwt), x[7:13]])  # fv
+    F = np.eye(13)
+    F[0:3, 7:10] = dt * np.eye(3)
+    F[3:7, 3:7] = np.array([[qwt[0], -qwt[1], -qwt[2], -qwt[3]], [qwt[1], qwt[0], qwt[3], -qwt[2]], [qwt[2], -qwt[3], qwt[0], qwt[1]],
+                            [qwt[3], qwt[2], -qwt[1], qwt[0]]])  # d(q * qwt) / dq, in dfv_by_dxv (:444-481)
+    ab = dq3_by_dq1(x[3:7]) @ dqomegadt_by_domega(x[10:13], dt)
+    F[3:7, 10:13] = ab
+    G = np.zeros((13, 6))
+    G[0:3, 0:3] = dt * np.eye(3)
+    G[3:7, 3:6] = ab
+    G[7:10, 0:3] = np.eye(3)
+    G[10:13, 3:6] = np.eye(3)
+    Q = G @ np.diag([(std_a * dt) ** 2] * 3 + [(std_alpha * dt) ** 2] * 3) @ G.T
+    xo = x.copy()
+    xo[0:13] = xv
+    Po = np.array(P, dtype=np.float64, order="F", copy=True)
+    Po[0:13, 0:13] = F @ P[0:13, 0:13] @ F.T + Q
+    Po[0:13, 13:] = F @ P[0:13, 13:]
+    Po[13:, 0:13] = P[13:, 0:13] @ F.T
+    return xo, Po
+
+
 def ekf_update(x, P, H, z, h, q4_int_exponent=True):
     """ExtendKF::update (src/ExtendKF.cpp:597-639), dense, general inverse."""
     if z.size == 0:

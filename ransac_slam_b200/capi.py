@@ -137,7 +137,8 @@ def make_camera(cam9):
 class Filter:
     """A batch of `batch` filters on one GPU (thin wrapper over the opaque rslam_filter handle)."""
 
-    def __init__(self, cam9, max_features, batch=1, device=0, quirks=Q_ALL, std_z=1.0, dedupe=True, n_hyp_initial=1000, std_a=0.007, std_alpha=0.007):
+    def __init__(self, cam9, max_features, batch=1, device=0, quirks=Q_ALL, std_z=1.0, dedupe=True, n_hyp_initial=1000, std_a=0.007, std_alpha=0.007,
+                 max_ellipse_eig=None):
         self.L = load()
         self.cam = make_camera(cam9)
         self.par = Params()
@@ -148,6 +149,8 @@ class Filter:
         self.par.std_alpha = std_alpha
         self.par.dedupe_hypotheses = int(dedupe)
         self.par.n_hyp_initial = n_hyp_initial
+        if max_ellipse_eig is not None:
+            self.par.max_ellipse_eig = max_ellipse_eig
         self.h = C.c_void_p()
         self.batch = batch
         self.max_features = max_features
@@ -251,10 +254,12 @@ class Filter:
         ic = np.ascontiguousarray(ic, dtype=np.uint8)
         self._ck(self.L.rslam_set_matches(self.h, b, _p(z), _p(ic)))
 
-    def set_image(self, img, b=0, share=False):
+    def set_image(self, img, b=0, share=False, cols=None):
+        """img: uint8 [rows, stride] on the host; the first `cols` (default: all) columns of each row are the image."""
         img = np.ascontiguousarray(img, dtype=np.uint8)
         self._keep = [img]
-        self._ck(self.L.rslam_set_image(self.h, b, _p(img), img.shape[0], img.shape[1], img.shape[1], int(share)))
+        cols = img.shape[1] if cols is None else cols
+        self._ck(self.L.rslam_set_image(self.h, b, _p(img), img.shape[0], cols, img.shape[1], int(share)))
 
     # -- stages -----------------------------------------------------------------------------------------------------
     def begin_frame(self):
@@ -265,6 +270,12 @@ class Filter:
 
     def search_ic_matches(self):
         self._ck(self.L.rslam_search_ic_matches(self.h))
+
+    def predict_measurements(self):
+        self._ck(self.L.rslam_predict_measurements(self.h))
+
+    def match(self):
+        self._ck(self.L.rslam_match(self.h))
 
     def ransac_hypotheses(self, u01, b=0):
         u = np.ascontiguousarray(u01, dtype=np.float64)

@@ -726,7 +726,7 @@ __global__ void __launch_bounds__(kSearchThreads) k_search(DevFilter* Fs, CamDev
     // predicted patch is zero when h is within half a patch of the border (src/Tracking.cpp:174-175,275) -> NaN scores -> no match
     if (!((h0 > kHalfPatch) && (h0 < (cam.nCols - kHalfPatch)) && (h1 > kHalfPatch) && (h1 < (cam.nRows - kHalfPatch)))) return;
     const int hsx = (int)ceil(2 * sqrt(S00)), hsy = (int)ceil(2 * sqrt(S11));
-    if (hsx > kMaxHalfSearch || hsy > kMaxHalfSearch) return;  // cannot happen while lmax < 100
+    if (hsx > kMaxHalfSearch || hsy > kMaxHalfSearch) return;  // cannot happen while lmax < max_eig <= 100 (rslam_create checks it)
     const int cx = (int)round(h0), cy = (int)round(h1);
     const int x_lo = cx - hsx, y_lo = cy - hsy;
     const int ncx = 2 * hsx + 1, ncy = 2 * hsy + 1;

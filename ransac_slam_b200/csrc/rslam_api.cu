@@ -76,8 +76,14 @@ struct rslam_filter {
     DevFilter* dF = nullptr;
     std::vector<void*> allocs;
     // shared buffers
-    unsigned char* d_images = nullptr;
+    unsigned char* d_images = nullptr;  // rslam_frame's host images (every call rebinds every filter)
     size_t image_cap = 0;
+    // rslam_set_image's host images: one buffer per filter and one for the image shared by the batch.  No call writes, moves or frees
+    // a buffer that a filter other than the one(s) it binds still reads.
+    std::vector<unsigned char*> si_img;
+    std::vector<size_t> si_cap;
+    unsigned char* si_shared = nullptr;
+    size_t si_shared_cap = 0;
     double* d_u01 = nullptr;
     size_t u01_cap = 0;
     // second staging set: rslam_prefetch_inputs copies the NEXT frame's host inputs into it on the copy stream while the current
@@ -398,6 +404,9 @@ const char* rslam_version(void) { return "rslam-b200 0.1 (sm_100a)"; }
 
 int rslam_create(const rslam_camera* cam, const rslam_params* par, int max_features, int batch, int device, rslam_filter** out) {
     if (!cam || !out || max_features < 1 || batch < 1) return fail(RSLAM_ERR_INVALID, "rslam_create: bad arguments");
+    // k_search stages windows of half-width <= kMaxHalfSearch = ceil(2 sqrt(100)); a larger gate would drop the features it lets through
+    if (par && !(par->max_ellipse_eig > 0.0 && par->max_ellipse_eig <= 100.0))
+        return fail(RSLAM_ERR_INVALID, "rslam_create: max_ellipse_eig = %g is not in (0, 100]", par->max_ellipse_eig);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();
@@ -558,6 +567,9 @@ int rslam_destroy(rslam_filter* f) {
     for (auto e : f->prof_pool) cudaEventDestroy(e);
     for (void* p : f->allocs) cudaFree(p);
     if (f->d_images) cudaFree(f->d_images);
+    for (unsigned char* p : f->si_img)
+        if (p) cudaFree(p);
+    if (f->si_shared) cudaFree(f->si_shared);
     if (f->d_u01) cudaFree(f->d_u01);
     if (f->pf_images) cudaFree(f->pf_images);
     if (f->pf_u01) cudaFree(f->pf_u01);
@@ -794,42 +806,45 @@ int rslam_set_matches(rslam_filter* f, int b, const double* z, const uint8_t* ic
     return RSLAM_OK;
 }
 
-static int set_images(rslam_filter* f, int b_first, int count, const uint8_t* gray, int rows, int cols, int stride, int share) {
-    // count == B (all filters) or 1 (filter b_first); share: one image for all
-    const bool dev = is_device_ptr(gray);
+// A host image is copied into a buffer of its own: filter b's (share == 0) or the batch's shared one (share != 0).  A buffer that
+// must grow is freed only while no filter outside this call's binding reads it: filter b's buffer is read by filter b alone, and the
+// shared buffer only by filters that a shared binding rebinds (all of them).
+static int set_images(rslam_filter* f, int b, const uint8_t* gray, int rows, int cols, int stride, int share) {
     const size_t per = (size_t)rows * stride;
-    const int nimg = share ? 1 : count;
-    const unsigned char* base = gray;
-    if (!dev) {
-        const size_t need = per * (share ? 1 : f->B);
-        if (need > f->image_cap) {
-            if (f->d_images) CK(cudaFree(f->d_images));
-            CK(cudaMalloc((void**)&f->d_images, need));
-            f->image_cap = need;
+    const unsigned char* img = gray;
+    if (!is_device_ptr(gray)) {
+        if (f->si_img.empty()) {
+            f->si_img.assign(f->B, nullptr);
+            f->si_cap.assign(f->B, 0);
         }
-        unsigned char* dst = f->d_images + (share ? 0 : per * b_first);
-        CK(cudaMemcpyAsync(dst, gray, per * nimg, cudaMemcpyHostToDevice, f->stream));
-        base = f->d_images;
-        if (!share && count == 1) base = f->d_images;  // per-filter slot addressing below
+        unsigned char*& buf = share ? f->si_shared : f->si_img[b];
+        size_t& cap = share ? f->si_shared_cap : f->si_cap[b];
+        if (per > cap) {
+            if (buf) CK(cudaFree(buf));  // synchronises with the work that still reads it
+            buf = nullptr;
+            cap = 0;
+            CK(cudaMalloc((void**)&buf, per));
+            cap = per;
+        }
+        CK(cudaMemcpyAsync(buf, gray, per, cudaMemcpyHostToDevice, f->stream));
+        img = buf;
     }
-    if (count == f->B || share) {
-        const unsigned char* b0 = dev ? gray : f->d_images;
-        LAUNCH(f, k_set_inputs, cdiv(f->B, 128), 128, 0, f->dF, f->B, b0, (long long)(share ? 0 : per), rows, cols, stride, 1, (const double*)nullptr, 0, 0);
-    f->bound_iper = -1;  // bound outside rslam_frame: its cache is stale
-    f->bound_nu = -1;
-        for (int b = 0; b < f->B; b++) {
-            f->hF[b].image = b0 + (share ? 0 : per * b);
-            f->hF[b].img_rows = rows;
-            f->hF[b].img_cols = cols;
-            f->hF[b].img_stride = stride;
+    if (share) {
+        LAUNCH(f, k_set_inputs, cdiv(f->B, 128), 128, 0, f->dF, f->B, img, 0LL, rows, cols, stride, 1, (const double*)nullptr, 0, 0);
+        f->bound_iper = -1;  // bound outside rslam_frame: its cache is stale
+        f->bound_nu = -1;
+        for (int k = 0; k < f->B; k++) {
+            f->hF[k].image = img;
+            f->hF[k].img_rows = rows;
+            f->hF[k].img_cols = cols;
+            f->hF[k].img_stride = stride;
         }
     } else {
-        DevFilter& D = f->hF[b_first];
-        D.image = dev ? gray : (f->d_images + per * b_first);
+        DevFilter& D = f->hF[b];
+        D.image = img;
         D.img_rows = rows;
         D.img_cols = cols;
         D.img_stride = stride;
-        (void)base;
         int rc = push_descr(f);
         if (rc) return rc;
     }
@@ -840,7 +855,7 @@ static int set_images(rslam_filter* f, int b_first, int count, const uint8_t* gr
 int rslam_set_image(rslam_filter* f, int b, const uint8_t* gray, int rows, int cols, int stride, int share) {
     if (!f || b < 0 || b >= f->B || !gray || rows <= 0 || cols <= 0 || stride < cols) return fail(RSLAM_ERR_INVALID, "rslam_set_image: bad arguments");
     CK(cudaSetDevice(f->device));
-    return set_images(f, b, 1, gray, rows, cols, stride, share);
+    return set_images(f, b, gray, rows, cols, stride, share);
 }
 
 int rslam_begin_frame(rslam_filter* f) {
