@@ -1151,6 +1151,27 @@ __device__ __forceinline__ bool gemm_setup(const DevFilter& F, int mode, int ste
     return true;
 }
 
+#ifdef RSLAM_PHASE_CLOCKS
+// Per-CTA timeline of filter 0's last syrk_P launch (record 0) and of its first trsm_outer launch (record 1), read by
+// rslam_debug_gemm_stamps: globaltimer at start and end, clock64 at start, after the first chunk has landed, after the main loop and
+// at the end, %smid, and the number of k-chunks.
+constexpr int kGemmStampCtas = 16384, kGemmStampFields = 8;
+__device__ unsigned long long g_gemm_stamps[2][kGemmStampCtas][kGemmStampFields];
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+__device__ __forceinline__ unsigned smid() {
+    unsigned s;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(s));
+    return s;
+}
+#define GEMM_STAMP(field, value) do { if (stamp__) stamp__[field] = (value); } while (0)
+#else
+#define GEMM_STAMP(field, value)
+#endif
+
 // In SYRK mode the product is taken over the n+1 rows of W: entries (n, c) of V V^T are (V y)[c] and update the state,
 //   x_k_k[c] = x0[c] + (V y)[c]   (x0 = x_k_km1 for the low-innovation update, x_k_k for the high-innovation one),
 // everything else is the covariance downdate P -= V V^T.
@@ -1180,36 +1201,67 @@ __global__ void __launch_bounds__(GemmCfg<BM, BN>::kThreads, GemmCfg<BM, BN>::kM
         ti = blockIdx.x % tm;
         tj = blockIdx.x / tm;
     }
+#ifdef RSLAM_PHASE_CLOCKS
+    const int rec__ = (mode & 0xff) == GEMM_SYRK_P ? 0 : ((mode & 0xff) == GEMM_TRSM_OUTER && step == 0 ? 1 : -1);
+    unsigned long long* stamp__ = rec__ >= 0 && blockIdx.z == 0 && blockIdx.x < kGemmStampCtas && threadIdx.x == 0 ? g_gemm_stamps[rec__][blockIdx.x] : nullptr;
+    GEMM_STAMP(0, globaltimer_ns());
+    GEMM_STAMP(2, clock64());
+    GEMM_STAMP(6, smid());
+    GEMM_STAMP(7, (g.K + GBK - 1) / GBK);
+#endif
     extern __shared__ __align__(16) double gsm[];
     double* As = gsm;                          // [stage][GBK][LDA]
     double* Bs = gsm + GSTAGES * GBK * LDA;    // [stage][GBK][LDB]
     const int m0 = ti * BM, n0 = tj * BN;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int wm0 = (warp % Cfg::kWM) * (MT * 8), wn0 = (warp / Cfg::kWM) * (NT * 8);
-    const int nkt = (g.K + GBK - 1) / GBK;
+    const int nkt = (g.K + GBK - 1) / GBK, nfull = g.K / GBK;  // k-chunks; those with all GBK columns inside K
     constexpr int A_CHUNKS = GBK * (BM / 2), B_CHUNKS = GBK * (BN / 2);
+    constexpr int A_PER = A_CHUNKS / THREADS, B_PER = B_CHUNKS / THREADS, KSTEPS = GBK / 4, CP_PER_KS = (A_PER + B_PER) / KSTEPS;
     static_assert(A_CHUNKS % THREADS == 0 && B_CHUNKS % THREADS == 0, "tile loads must divide evenly");
+    static_assert(THREADS % (BM / 2) == 0 && THREADS % (BN / 2) == 0, "a thread copies the same rows in every k-row it serves");
+    static_assert((A_PER + B_PER) % KSTEPS == 0, "copies spread evenly over the k-steps of a chunk");
+    constexpr int A_KSTRIDE = THREADS / (BM / 2), B_KSTRIDE = THREADS / (BN / 2);  // k-rows between a thread's successive copies
 
-    auto load_stage = [&](int stage, int kt) {
-        const int k0 = kt * GBK;
+    // Copy slots: a thread's 16-byte copies of a chunk all read the same two rows of A (of B), in k-rows kc0, kc0 + KSTRIDE, ...
+    // The row test and the source pointers are set up once per tile; per chunk the pointers advance by GBK columns.  A row past
+    // M (N) is zero-filled from a pointer kept on row 0, which stays inside the operand on every chunk that is not the last.
+    const int a_kc = tid / (BM / 2), a_r = 2 * (tid % (BM / 2));
+    const int b_kc = tid / (BN / 2), b_r = 2 * (tid % (BN / 2));
+    const bool a_ok = m0 + a_r < g.M, b_ok = n0 + b_r < g.N;
+    const double* pa = g.A + (a_ok ? m0 + a_r : 0) + (size_t)a_kc * g.lda;  // the next chunk to load
+    const double* pb = g.B + (b_ok ? n0 + b_r : 0) + (size_t)b_kc * g.ldb;
+    const size_t a_step = (size_t)A_KSTRIDE * g.lda, b_step = (size_t)B_KSTRIDE * g.ldb;
+    const size_t a_chunk = (size_t)GBK * g.lda, b_chunk = (size_t)GBK * g.ldb;
+    double* const a_dst = As + a_kc * LDA + a_r;
+    double* const b_dst = Bs + b_kc * LDB + b_r;
+    auto copy = [&](int stage, int i) {  // copy i of this thread for the chunk at pa / pb, a full chunk
+        if (i < A_PER)
+            cp_async16(a_dst + (stage * GBK + i * A_KSTRIDE) * LDA, pa + i * a_step, a_ok);
+        else
+            cp_async16(b_dst + (stage * GBK + (i - A_PER) * B_KSTRIDE) * LDB, pb + (i - A_PER) * b_step, b_ok);
+    };
+    auto copy_last = [&](int stage, int kleft) {  // the chunk that ends past K: columns >= K zero-filled, like rows >= M
 #pragma unroll
-        for (int it = 0; it < A_CHUNKS / THREADS; it++) {
-            const int ch = tid + it * THREADS;
-            const int kc = ch / (BM / 2), r2 = ch % (BM / 2);
-            const int row = m0 + 2 * r2, col = k0 + kc;
-            const bool v = (row < g.M) && (col < g.K);
-            const double* src = v ? (g.A + row + (size_t)col * g.lda) : g.A;
-            cp_async16(&As[(stage * GBK + kc) * LDA + 2 * r2], src, v);
+        for (int i = 0; i < A_PER; i++) {
+            const bool v = a_ok && a_kc + i * A_KSTRIDE < kleft;
+            cp_async16(a_dst + (stage * GBK + i * A_KSTRIDE) * LDA, v ? pa + i * a_step : g.A, v);
         }
 #pragma unroll
-        for (int it = 0; it < B_CHUNKS / THREADS; it++) {
-            const int ch = tid + it * THREADS;
-            const int kc = ch / (BN / 2), r2 = ch % (BN / 2);
-            const int row = n0 + 2 * r2, col = k0 + kc;
-            const bool v = (row < g.N) && (col < g.K);
-            const double* src = v ? (g.B + row + (size_t)col * g.ldb) : g.B;
-            cp_async16(&Bs[(stage * GBK + kc) * LDB + 2 * r2], src, v);
+        for (int i = 0; i < B_PER; i++) {
+            const bool v = b_ok && b_kc + i * B_KSTRIDE < kleft;
+            cp_async16(b_dst + (stage * GBK + i * B_KSTRIDE) * LDB, v ? pb + i * b_step : g.B, v);
         }
+    };
+    auto load_stage = [&](int stage, int kt) {  // whole chunk kt at once (prologue, and the last chunk when it ends past K)
+        if (kt < nfull) {
+#pragma unroll
+            for (int i = 0; i < A_PER + B_PER; i++) copy(stage, i);
+        } else if (kt < nkt) {
+            copy_last(stage, g.K - kt * GBK);
+        }
+        pa += a_chunk;
+        pb += b_chunk;
     };
 
     double acc[MT][NT][2];
@@ -1218,36 +1270,62 @@ __global__ void __launch_bounds__(GemmCfg<BM, BN>::kThreads, GemmCfg<BM, BN>::kM
 #pragma unroll
         for (int b = 0; b < NT; b++) acc[a][b][0] = acc[a][b][1] = 0.0;
 
+    // One chunk of DMMA work.  The fragments of k-step ks + 1 are loaded while the DMMAs of k-step ks issue, and `copies(ks)` issues
+    // that k-step's share of the next stage's copies between them, so neither the copy issue nor the first fragment loads of a
+    // k-step sit in front of the tensor pipe as one block.  Every accumulator still takes its DMMAs in ascending k.
+    const int frag_a = (lane & 3) * LDA + wm0 + (lane >> 2), frag_b = (lane & 3) * LDB + wn0 + (lane >> 2);
+    auto compute = [&](const double* as, const double* bs, auto&& copies) {
+        double af[2][MT], bf[2][NT];
+#pragma unroll
+        for (int mt = 0; mt < MT; mt++) af[0][mt] = as[frag_a + mt * 8];
+#pragma unroll
+        for (int nt = 0; nt < NT; nt++) bf[0][nt] = bs[frag_b + nt * 8];
+#pragma unroll
+        for (int ks = 0; ks < KSTEPS; ks++) {
+            const int cur = ks & 1;
+            if (ks + 1 < KSTEPS) {
+#pragma unroll
+                for (int mt = 0; mt < MT; mt++) af[cur ^ 1][mt] = as[frag_a + (ks + 1) * 4 * LDA + mt * 8];
+#pragma unroll
+                for (int nt = 0; nt < NT; nt++) bf[cur ^ 1][nt] = bs[frag_b + (ks + 1) * 4 * LDB + nt * 8];
+            }
+            copies(ks);
+#pragma unroll
+            for (int mt = 0; mt < MT; mt++)
+#pragma unroll
+                for (int nt = 0; nt < NT; nt++) dmma8x8x4(acc[mt][nt][0], acc[mt][nt][1], af[cur][mt], bf[cur][nt]);
+        }
+    };
+
 #pragma unroll
     for (int s = 0; s < GSTAGES - 1; s++) {
-        if (s < nkt) load_stage(s, s);
+        load_stage(s, s);
         cp_async_commit();
     }
     for (int kt = 0; kt < nkt; kt++) {
         cp_async_wait<GSTAGES - 2>();
         __syncthreads();
-        {
-            const int nk = kt + GSTAGES - 1;
-            if (nk < nkt) load_stage(nk % GSTAGES, nk);
-            cp_async_commit();
-        }
+#ifdef RSLAM_PHASE_CLOCKS
+        if (kt == 0) GEMM_STAMP(3, clock64());
+#endif
+        const int nk = kt + GSTAGES - 1, ns = nk % GSTAGES;  // the chunk loaded during this one, into the stage read last time
         const double* as = As + (kt % GSTAGES) * GBK * LDA;
         const double* bs = Bs + (kt % GSTAGES) * GBK * LDB;
+        if (nk < nfull) {
+            compute(as, bs, [&](int ks) {
 #pragma unroll
-        for (int ks = 0; ks < GBK / 4; ks++) {
-            const int krow = ks * 4 + (lane & 3);
-            double af[MT], bf[NT];
-#pragma unroll
-            for (int mt = 0; mt < MT; mt++) af[mt] = as[krow * LDA + wm0 + mt * 8 + (lane >> 2)];
-#pragma unroll
-            for (int nt = 0; nt < NT; nt++) bf[nt] = bs[krow * LDB + wn0 + nt * 8 + (lane >> 2)];
-#pragma unroll
-            for (int mt = 0; mt < MT; mt++)
-#pragma unroll
-                for (int nt = 0; nt < NT; nt++) dmma8x8x4(acc[mt][nt][0], acc[mt][nt][1], af[mt], bf[nt]);
+                for (int c = 0; c < CP_PER_KS; c++) copy(ns, ks * CP_PER_KS + c);
+            });
+            pa += a_chunk;
+            pb += b_chunk;
+        } else {
+            load_stage(ns, nk);
+            compute(as, bs, [](int) {});
         }
+        cp_async_commit();
     }
     cp_async_wait<0>();
+    GEMM_STAMP(4, clock64());
     const bool syrk = (mode & 0xff) == GEMM_SYRK_P;
     const int xrow = syrk ? F.n : -1;
     const double* x0 = ((mode >> 8) & 0xff) ? F.x_kk : F.x_km1;
@@ -1293,7 +1371,10 @@ __global__ void __launch_bounds__(GemmCfg<BM, BN>::kThreads, GemmCfg<BM, BN>::kM
                 }
         }
     }
+    GEMM_STAMP(5, clock64());
+    GEMM_STAMP(1, globaltimer_ns());
 }
+#undef GEMM_STAMP
 
 // ---- U6s: covariance downdate for SMALL innovation dimension (k <= 256: the 100-feature and batched-filter configurations) -----
 // With K this small a 64 x 64 tile is a handful of k-steps, so the one-tile-per-CTA GEMM above spends most of its life in the

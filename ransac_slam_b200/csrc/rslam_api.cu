@@ -1211,6 +1211,21 @@ extern "C" int rslam_debug_sup_clocks(unsigned long long* out8) {
     return 0;
 }
 #endif
+#ifdef RSLAM_PHASE_CLOCKS
+// per-CTA timeline of k_gemm_dmma (record 0: the last syrk_P launch, 1: the first trsm_outer launch; filter 0): up to max_ctas
+// rows of 8 values, zeroed after the read
+extern "C" int rslam_debug_gemm_stamps(int record, unsigned long long* out, int max_ctas) {
+    if (record < 0 || record > 1 || !out || max_ctas <= 0) return -1;
+    const int n = std::min(max_ctas, rslam::kGemmStampCtas);
+    const size_t row = sizeof(unsigned long long) * rslam::kGemmStampFields, off = (size_t)record * rslam::kGemmStampCtas * row;
+    cudaDeviceSynchronize();
+    if (cudaMemcpyFromSymbol(out, rslam::g_gemm_stamps, n * row, off) != cudaSuccess) return -1;
+    void* p = nullptr;
+    if (cudaGetSymbolAddress(&p, rslam::g_gemm_stamps) != cudaSuccess || cudaMemset((char*)p + off, 0, rslam::kGemmStampCtas * row) != cudaSuccess) return -1;
+    cudaDeviceSynchronize();
+    return n;
+}
+#endif
 // diagnostics: the 32-double scratch block of filter b (phase clocks when built with -DRSLAM_PHASE_CLOCKS)
 int rslam_debug_scratch(rslam_filter* f, int b, double* out32) {
     if (!f || b < 0 || b >= f->B || !out32) return fail(RSLAM_ERR_INVALID, "rslam_debug_scratch: bad arguments");
