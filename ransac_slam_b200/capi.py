@@ -138,7 +138,7 @@ class Filter:
     """A batch of `batch` filters on one GPU (thin wrapper over the opaque rslam_filter handle)."""
 
     def __init__(self, cam9, max_features, batch=1, device=0, quirks=Q_ALL, std_z=1.0, dedupe=True, n_hyp_initial=1000, std_a=0.007, std_alpha=0.007,
-                 max_ellipse_eig=None):
+                 max_ellipse_eig=None, p_spurious_free=None):
         self.L = load()
         self.cam = make_camera(cam9)
         self.par = Params()
@@ -151,6 +151,8 @@ class Filter:
         self.par.n_hyp_initial = n_hyp_initial
         if max_ellipse_eig is not None:
             self.par.max_ellipse_eig = max_ellipse_eig
+        if p_spurious_free is not None:
+            self.par.p_spurious_free = p_spurious_free
         self.h = C.c_void_p()
         self.batch = batch
         self.max_features = max_features

@@ -957,7 +957,7 @@ __device__ __forceinline__ bool support_pair_inlier(const DevFilter& F, const Ca
         const double f = rd + cam.k1 * (rd2 * rd) + cam.k2 * (rd4 * rd) - ru;
         const double fp = 1 + 3 * cam.k1 * rd2 + 5 * cam.k2 * rd4;
         const double rn = fma(-f, fast_rcp(fp), rd);
-        const bool same = !(rn != rd) || !live;  // NaN counts as settled
+        const bool same = !(rn != rd) || !live;  // a NaN lane never settles: rn != rd is true for NaN, so it runs all 10 steps
         rd = rn;
         if (__all_sync(0xffffffffu, same)) break;
     }
