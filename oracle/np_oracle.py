@@ -108,6 +108,79 @@ def jacobian_H(cam, x, types, i, h_i):
     return H
 
 
+def undistort_fm(cam, uv):  # src/ExtendKF.cpp:266-285 ; uv: (m, 2)
+    k1, k2, _, _, Cx, Cy, _, dx, dy = cam
+    xd = (uv[:, 0] - Cx) * dx
+    yd = (uv[:, 1] - Cy) * dy
+    rd2 = xd**2 + yd**2
+    D = 1 + k1 * rd2 + k2 * rd2**2
+    return np.stack([xd * D / dx + Cx, yd * D / dy + Cy], axis=1)
+
+
+def xyz_w_for_warp(x, types, i):
+    """The XYZ_w that Tracking::search_IC_matches hands pred_patch_fc for feature i (src/Tracking.cpp:47-66): the point of the last
+    inverse-depth feature at or before i; a cartesian feature does not recompute it (quirk Q3), so one that precedes every
+    inverse-depth feature gets the initial zeros."""
+    X = np.zeros(3)
+    off = 13
+    for k in range(i + 1):
+        if types[k] == 0:
+            y = x[off:off + 6]
+            X = y[0:3] + (1.0 / y[5]) * np.array([np.cos(y[4]) * np.sin(y[3]), -np.sin(y[4]), np.cos(y[4]) * np.cos(y[3])])
+            off += 6
+        else:
+            off += 3
+    return X
+
+
+def pred_patch_maps(cam, x, h, XYZ_w, r_init, R_init, uv_init, half_pred=6, half_init=20):
+    """Tracking::pred_patch_fc (src/Tracking.cpp:164-278) up to the cv::remap call, for one feature predicted at h (distorted pixel)
+    from the prior x: R_init (3 x 3, as uploaded), r_init and uv_init are what Map::initialize_a_features stored, XYZ_w as
+    xyz_w_for_warp.  Quirks kept: Q11 (the -1 in the patch offset), Q12 (the translation enters as R r), Q13 (cv::Range truncates).
+    Returns (xs, ys, ok, mapx, mapy, c2): the window origin in the current image, ok = -1 if h is within half a patch of the border,
+    0 if the truncated window is not 13 x 13 (both give the zero patch), 1 otherwise; mapx / mapy (13 x 13, row = y) are the
+    coordinates in the 41 x 41 initial patch that cv::remap samples (None unless ok == 1); c2 is the window centre before truncation
+    (None if ok == -1)."""
+    k1, k2, nRows, nCols, Cx, Cy, f, dx, dy = cam
+    n_len = 2 * half_pred + 1
+    if not (half_pred < h[0] < nCols - half_pred and half_pred < h[1] < nRows - half_pred):
+        return 0, 0, -1, None, None, None
+
+    def homog4(R, r):  # [R 0; 0 1] [I r; 0 1]
+        H4 = np.eye(4)
+        H4[:3, :3] = R
+        H4[:3, 3] = R @ r
+        return H4
+
+    Hpf = homog4(np.asarray(R_init, float).reshape(3, 3), np.asarray(r_init, float))
+    Hpfi = np.linalg.inv(Hpf)
+    Hkk = Hpfi @ homog4(q2r(x[3:7]), x[0:3])
+    n1 = np.array([uv_init[0] - Cx, uv_init[1] - Cy, -f / dx])
+    n = n1 / np.linalg.norm(n1)
+    nt4 = Hkk @ np.array([h[0] - Cx, h[1] - Cy, -f / dx, 1.0])
+    nt = nt4[:3] / nt4[3]
+    ns = n + nt / np.linalg.norm(nt)
+    n = ns / np.linalg.norm(ns)
+    Xk = Hpfi @ np.append(XYZ_w, 1.0)
+    d = -(n @ (Xk[:3] / Xk[3]))
+    K = np.array([[f / dx, 0, Cx], [0, f / dy, Cy], [0, 0, 1.0]])
+    Hm = K @ (Hkk[:3, :3] - np.outer(Hkk[:3, 3], n) / d) @ np.linalg.inv(K)
+    w = np.linalg.solve(Hm, np.append(undistort_fm(cam, np.array([uv_init]))[0], 1.0))
+    c2 = distort_fm(cam, np.array([w[:2] / w[2]]))[0]
+    xs, xe = int(c2[0] - half_pred), int(c2[0] + half_pred)  # int() truncates toward zero like cv::Range(double, double)
+    ys, ye = int(c2[1] - half_pred), int(c2[1] + half_pred)
+    if xe - xs + 1 != n_len or ye - ys + 1 != n_len:
+        return xs, ys, 0, None, None, c2
+    gy, gx = np.mgrid[ys:ys + n_len, xs:xs + n_len].astype(float)
+    und = undistort_fm(cam, np.stack([gx.ravel(), gy.ravel()], axis=1))
+    p = Hm @ np.vstack([und.T, np.ones(und.shape[0])])
+    with np.errstate(divide="ignore", invalid="ignore"):
+        c1 = distort_fm(cam, np.stack([p[0] / p[2], p[1] / p[2]], axis=1))
+    mapx = c1[:, 0].reshape(n_len, n_len) - (uv_init[0] - half_init - 1)
+    mapy = c1[:, 1].reshape(n_len, n_len) - (uv_init[1] - half_init - 1)
+    return xs, ys, 1, mapx, mapy, c2
+
+
 def v2q(v, eps=2.220446049250313e-16):  # src/ExtendKF.cpp:428-443 (quirk Q14: the zero quaternion below eps)
     theta = np.sqrt(v @ v)
     if theta < eps:

@@ -20,6 +20,7 @@
 // Quirks of the reference that change results are reproduced (SURVEY.md A.3) behind named switches that default
 // to reference behaviour.
 #include <cfenv>
+#include <climits>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -381,7 +382,9 @@ static Mat PHt(const Filter& F, int i, const Mat& P) {
 // cv::remap(src CV_32F, map1/map2 CV_32F, INTER_LINEAR, BORDER_CONSTANT, 0): map coordinates are quantised to 1/32 px
 // (sx = cvRound(32*x) round-half-even, ix = sx>>5, fx = sx&31), weights (1-fx/32)(1-fy/32) ... as float; out-of-range
 // taps read the border value 0.
-static inline int cv_round(double v) { return (int)std::nearbyint(v); }  // default rounding mode: to nearest even
+// default rounding mode: to nearest even.  NaN and values outside int give INT_MIN, what cvRound's cvtsd2si returns on x86 (the
+// cast alone would be undefined behaviour); remap then reads the border value
+static inline int cv_round(double v) { return (v >= -2147483648.0 && v < 2147483648.0) ? (int)std::nearbyint(v) : INT_MIN; }
 static Mat cv_remap_linear_const0(const Mat& src, const Mat& mapx, const Mat& mapy) {
     int orow = mapx.rows(), ocol = mapx.cols();
     Mat dst(orow, ocol);

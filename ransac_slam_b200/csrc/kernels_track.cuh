@@ -683,7 +683,9 @@ __global__ void __launch_bounds__(192) k_pred_patch(DevFilter* Fs, CamDev cam) {
     double c1u, c1v;
     distort_exact_dev(cam, w0 / w2, w1 / w2, c1u, c1v);
     const float mx = (float)(c1u - (uvf0 - 20 - 1)), my = (float)(c1v - (uvf1 - 20 - 1));
-    const int sx = __float2int_rn(mx * 32.0f), sy = __float2int_rn(my * 32.0f);
+    // A pixel on the homography's vanishing line (w2 == 0) has a NaN map coordinate.  cvRound(NaN) is INT_MIN on x86, so cv::remap
+    // reads the border value there; __float2int_rn(NaN) is 0, which would read the patch's corner instead.
+    const int sx = isnan(mx) ? INT_MIN : __float2int_rn(mx * 32.0f), sy = isnan(my) ? INT_MIN : __float2int_rn(my * 32.0f);
     const int ix = sx >> 5, iy = sy >> 5;
     const float fx = (float)(sx & 31) / 32.0f, fy = (float)(sy & 31) / 32.0f;
     const float w00 = (1.f - fy) * (1.f - fx), w01 = (1.f - fy) * fx, w10 = fy * (1.f - fx), w11 = fy * fx;
