@@ -258,34 +258,37 @@ __device__ __forceinline__ double map_quad(const double* cr, const double* cc, i
     return v;
 }
 
-// P' = T P T^T + E and x' = T x, out of place.  grid (ceil(n_new / 256), n_new): thread per entry, blockIdx.y = column.
+// P' = T P T^T + E and x' = T x, out of place.  grid (ceil(n_new / 256), min(n_new, 65535)): thread per entry; a CTA row takes
+// columns blockIdx.y, blockIdx.y + gridDim.y, ... (gridDim.y is capped at 65535, and a map may have more state rows than that).
 __global__ void __launch_bounds__(256) k_map_xform(DevFilter* Fs, int b, MapXform xf, const double* scratch, double* Pdst, double* xdst) {
     const DevFilter& F = Fs[b];
-    const int r = blockIdx.x * blockDim.x + threadIdx.x, c = blockIdx.y;
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= xf.n_new) return;
     const size_t ld = F.ldp;
     const double* P = F.P;
     const double* C = scratch + kMapC;
     const bool rs = r >= xf.sp_at && r < xf.sp_at + xf.sp_cnt;
-    const bool cs = c >= xf.sp_at && c < xf.sp_at + xf.sp_cnt;
-    double v;
-    if (!rs && !cs) {
-        v = P[map_old_row(xf, r) + (size_t)map_old_row(xf, c) * ld];
-    } else if (rs && !cs) {
-        const double* col = P + (size_t)map_old_row(xf, c) * ld + xf.src_at;
-        v = map_comb(C + (r - xf.sp_at) * xf.src_cnt, xf.src_cnt, [&](int k) { return col[k]; });
-    } else if (!rs && cs) {
-        const double* row = P + map_old_row(xf, r) + (size_t)xf.src_at * ld;
-        v = map_comb(C + (c - xf.sp_at) * xf.src_cnt, xf.src_cnt, [&](int k) { return row[(size_t)k * ld]; });
-    } else {
-        // evaluated for the lower-triangle position and mirrored, so that P stays exactly symmetric (the library's invariant)
-        const int rr = r > c ? r : c, c2 = r > c ? c : r;
-        const double* S = P + xf.src_at + (size_t)xf.src_at * ld;
-        v = map_quad(C + (rr - xf.sp_at) * xf.src_cnt, C + (c2 - xf.sp_at) * xf.src_cnt, xf.src_cnt, [&](int l, int k) { return S[l + (size_t)k * ld]; });
-        v += scratch[kMapE + (rr - xf.sp_at) * 6 + (c2 - xf.sp_at)];
+    for (int c = blockIdx.y; c < xf.n_new; c += gridDim.y) {
+        const bool cs = c >= xf.sp_at && c < xf.sp_at + xf.sp_cnt;
+        double v;
+        if (!rs && !cs) {
+            v = P[map_old_row(xf, r) + (size_t)map_old_row(xf, c) * ld];
+        } else if (rs && !cs) {
+            const double* col = P + (size_t)map_old_row(xf, c) * ld + xf.src_at;
+            v = map_comb(C + (r - xf.sp_at) * xf.src_cnt, xf.src_cnt, [&](int k) { return col[k]; });
+        } else if (!rs && cs) {
+            const double* row = P + map_old_row(xf, r) + (size_t)xf.src_at * ld;
+            v = map_comb(C + (c - xf.sp_at) * xf.src_cnt, xf.src_cnt, [&](int k) { return row[(size_t)k * ld]; });
+        } else {
+            // evaluated for the lower-triangle position and mirrored, so that P stays exactly symmetric (the library's invariant)
+            const int rr = r > c ? r : c, c2 = r > c ? c : r;
+            const double* S = P + xf.src_at + (size_t)xf.src_at * ld;
+            v = map_quad(C + (rr - xf.sp_at) * xf.src_cnt, C + (c2 - xf.sp_at) * xf.src_cnt, xf.src_cnt, [&](int l, int k) { return S[l + (size_t)k * ld]; });
+            v += scratch[kMapE + (rr - xf.sp_at) * 6 + (c2 - xf.sp_at)];
+        }
+        Pdst[r + (size_t)c * ld] = v;
+        if (c == 0) xdst[r] = rs ? scratch[kMapX + (r - xf.sp_at)] : F.x_kk[map_old_row(xf, r)];
     }
-    Pdst[r + (size_t)c * ld] = v;
-    if (c == 0) xdst[r] = rs ? scratch[kMapX + (r - xf.sp_at)] : F.x_kk[map_old_row(xf, r)];
 }
 
 // ---- feature initialisation (SURVEY 8f row 4): cv::FAST (TYPE_9_16, non-maximum suppression) + the "features in the box" test ----

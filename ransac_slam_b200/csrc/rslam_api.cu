@@ -1443,7 +1443,7 @@ int map_sync_layout(rslam_filter* f, int b) {
 // run P' = T P T^T + E, x' = T x into the spare buffers and swap them in
 int map_apply(rslam_filter* f, int b, const MapXform& xf) {
     DevFilter& D = f->hF[b];
-    LAUNCH(f, k_map_xform, dim3(cdiv(xf.n_new, 256), xf.n_new), 256, 0, f->dF, b, xf, (const double*)f->map_coef, f->map_P, f->map_x);
+    LAUNCH(f, k_map_xform, dim3(cdiv(xf.n_new, 256), std::min(xf.n_new, 65535)), 256, 0, f->dF, b, xf, (const double*)f->map_coef, f->map_P, f->map_x);
     std::swap(D.P, f->map_P);
     std::swap(D.x_kk, f->map_x);
     D.n = xf.n_new;
